@@ -65,7 +65,13 @@ def parse():
     ap.add_argument("--ref-budget", type=float, default=200.0, help="seconds for the whole --impl reference run")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--extra-opts", default="", help="more -geneo_* / -els2_* options, space separated")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step returned (solution x, its / rnorm / reason) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     graph = a.kind == "graph"
     a.size = a.size or (1000000 if graph else 200)
     a.partition = a.partition or ("metis" if graph else "box")
@@ -305,6 +311,21 @@ def build_problem(a, g, dist, rank, world, edge, partition):
     return prob, layout, {"gen_s": t1 - t0, "part_decomp_s": t2 - t1}
 
 
+DUMP_X_MAX = 1 << 21  # rows of x written by --dump-outputs: 2 x 16 MB with their ids
+
+
+def dump_outputs(d, x, r):
+    """The result of the last timed step as float64 .npy files: x (the solution; above DUMP_X_MAX rows a fixed seeded sample
+    of them, whose row ids are x_index) and ksp = [iterations, rnorm, reason]."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    n = x.shape[0]
+    idx = np.arange(n) if n <= DUMP_X_MAX else np.sort(np.random.default_rng(0).choice(n, DUMP_X_MAX, replace=False))
+    np.save(os.path.join(d, "x.npy"), x[idx])
+    np.save(os.path.join(d, "x_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(d, "ksp.npy"), np.array([r["its"], r["rnorm"], r["reason"]], dtype=np.float64))
+
+
 def run_b200(a):
     import numpy as np
     import torch
@@ -315,6 +336,8 @@ def run_b200(a):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device -- the product has no CPU fallback")
+    if a.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs writes the solution of a single process; run it on one GPU")
     torch.cuda.set_device(local)
     tdist = None
     if world > 1:
@@ -388,6 +411,8 @@ def run_b200(a):
     kms, klaunch = pc.kernel_time()
     assert r["reason"] > 0, "KSP did not converge: %s" % r["reason_name"]
     err = float((x[:n_own] - ones[:n_own]).abs().max() / n)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, x[:n_own].cpu().numpy(), r)
     phases = {k: pc.timers()[k] for k in ("lvl1SetupMinv", "lvl2SetupSyl", "lvl2SetupEig", "lvl2SetupZ", "lvl2SetupE")}
     info = pc.info()
 

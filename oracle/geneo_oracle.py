@@ -137,10 +137,15 @@ def read_rhs_file(path: str, n: int) -> np.ndarray:
 def ref_generator(kind: str, args: str) -> Mesh:
     """Run the reference's OWN generator (oracle/_ref/libgen<kind>.so, built from tst/<kind>/*.cpp) -- the
     `--inpLibA L A` path of src/geneo4PETSc.cpp:75-96."""
-    lib = _shim()
     path = os.path.join(_HERE, "_ref", "libgen%s.so" % kind)
     if not os.path.exists(path):
         raise FileNotFoundError(path + " (run `make -C oracle ref` where /root/reference exists)")
+    return plugin_input(path, args)
+
+
+def plugin_input(path: str, args: str) -> Mesh:
+    """The mesh of any library exporting the reference's getInput() plug-in ABI, called with `args`."""
+    lib = _shim()
     ne, nn = ctypes.c_uint32(), ctypes.c_uint32()
     p_ptr, p_idx = ctypes.POINTER(ctypes.c_uint32)(), ctypes.POINTER(ctypes.c_uint32)()
     p_val = ctypes.POINTER(ctypes.c_double)()
@@ -148,7 +153,7 @@ def ref_generator(kind: str, args: str) -> Mesh:
     rc = lib.oracle_get_input(path.encode(), args.encode(), ctypes.byref(ne), ctypes.byref(nn), ctypes.byref(p_ptr),
                               ctypes.byref(p_idx), ctypes.byref(n_idx), ctypes.byref(p_val), ctypes.byref(n_val))
     if rc != 0:
-        raise RuntimeError("reference generator failed")
+        raise RuntimeError("getInput of %s failed" % path)
     elem_ptr = np.ctypeslib.as_array(p_ptr, shape=(ne.value + 1,)).astype(np.int64)
     elem_idx = np.ctypeslib.as_array(p_idx, shape=(max(n_idx.value, 1),))[: n_idx.value].astype(np.int64)
     mat_val = np.ctypeslib.as_array(p_val, shape=(max(n_val.value, 1),))[: n_val.value].copy()

@@ -1,11 +1,13 @@
-"""bench.py contract checks that need no GPU: the reference arm (CPU restatement on the host cores) prints one JSON line whose
-`config.workload` names the size it REALLY ran, with the keys the driver reads; box grids of the multi-GPU layout."""
+"""bench.py contract checks.  Without a GPU: the reference arm (CPU restatement on the host cores) prints one JSON line whose
+`config.workload` names the size it REALLY ran, with the keys a reader of the result line needs; box grids of the multi-GPU layout; argument
+checks.  On the GPU: --dump-outputs."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -45,3 +47,31 @@ def test_box_grids_cover_every_rank_evenly():
                     b3 = (b % K[0], (b // K[0]) % K[1], b // (K[0] * K[1]))
                     first = [-(-b3[a] * 97 // K[a]) for a in range(3)]
                     assert all(lo[a] <= first[a] < hi[a] for a in range(3))
+
+
+def test_bench_rejects_runs_without_timed_steps():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_solution(tmp_path):
+    """--dump-outputs DIR: x of the last timed step (all rows at this size, ids in x_index) and [its, rnorm, reason], float64;
+    the same arguments give the same inputs, so two runs agree to the solver's tolerance."""
+    runs = []
+    for k in range(2):
+        d = tmp_path / ("run%d" % k)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--size", "16", "--steps", "2", "--warmup", "1",
+                            "--e2e-steps", "1", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=900, cwd=tmp_path)
+        assert r.returncode == 0, r.stderr[-800:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+        runs.append({name: np.load(d / (name + ".npy")) for name in ("x", "x_index", "ksp")})
+    for out in runs:
+        assert all(v.dtype == np.float64 for v in out.values())
+        np.testing.assert_array_equal(out["x_index"], np.arange(16 ** 3))
+        # b = A (1..N); CG stops at 1e-5 on the preconditioned residual: ~2e-3 absolute error on every row
+        assert np.linalg.norm(out["x"] - (out["x_index"] + 1.0)) <= 1e-4 * np.linalg.norm(out["x_index"] + 1.0)
+        assert out["ksp"][0] >= 1 and out["ksp"][2] > 0
+    np.testing.assert_allclose(runs[0]["x"], runs[1]["x"], rtol=1e-8)
+    assert runs[0]["ksp"][0] == runs[1]["ksp"][0]

@@ -270,22 +270,23 @@ def test_chain_pairs_cover_every_update_exactly_once():
     assert np.linalg.norm(a @ x - b) <= 1e-10 * np.linalg.norm(b)
 
 
-def test_cli_loads_getinput_plugins_like_the_reference():
+def test_cli_loads_getinput_plugins_like_the_reference(tmp_path):
     """--inpLibA L A: the driver dlopens any library exporting the reference's getInput() (src/geneo4PETSc.cpp:75-96).  Here L
-    is the reference's OWN graph generator (oracle/_ref/libgengraph.so, built from tst/graph/graph.cpp); the local matrices
-    the driver dumps must be those of the oracle's decomposition of the same mesh."""
+    is tests/plugins/gen_web.cpp, an irregular graph Laplacian; the local matrices the driver dumps must be those of the
+    oracle's decomposition of the mesh the same library returns."""
     import os
     import subprocess
     from tests._cases import parse_driver_log
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    lib = os.path.join(root, "oracle", "_ref", "libgengraph.so")
-    if not os.path.exists(lib):
-        pytest.skip("oracle/_ref/libgengraph.so not built (needs /root/reference at build time)")
-    args = "--size 100 --level 2 --noGround --inpEps 0.0001"
+    lib = str(tmp_path / "libgenweb.so")
+    cxx = "/usr/bin/g++" if os.access("/usr/bin/g++", os.X_OK) else "g++"  # shared libstdc++: std::vector crosses dlopen (oracle/Makefile)
+    subprocess.run([cxx, "-O2", "-std=c++11", "-fPIC", "-shared", "-o", lib, os.path.join(root, "tests", "plugins", "gen_web.cpp")],
+                   check=True)
+    args = "--size 300 --inpEps 0.0001"
     r = subprocess.run([os.path.join(root, "geneo4petsc_b200", "geneo4PETSc"), "--inpLibA", lib, args.replace(" ", "#"), "--nbPart", "3",
                         "--verbose", "2", "-pc_type", "geneo"], capture_output=True, text=True, timeout=120)
     got = parse_driver_log(r.stdout)
-    mesh = go.ref_generator("graph", args)
+    mesh = go.plugin_input(lib, args)
     p = g.Problem().set_mesh(mesh.nb_node, mesh.elem_ptr, mesh.elem_idx, mesh.mat_val).decompose(3, True, 0)
     ep, npart = p.partition()
     dec = go.decompose(mesh, 3, ep, npart, True, 0)
