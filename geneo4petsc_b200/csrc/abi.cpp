@@ -677,6 +677,9 @@ int geneo_host_sym_eig(int n, double* a, double* w) { ABI_TRY ABI_REQ(a && w && 
 
 int geneo_microbench(int kind, int n, int reps, double result[2]) {
   ABI_TRY
+  // checked before anything touches the device: a bad kind allocates no synthetic forest
+  ABI_REQ(kind < 100 || kind % 100 == 1 || kind % 100 == 8 || kind % 100 == 16,
+          "microbench kind 100*nlev + nr: nr must be 1, 8 or 16");
   require_device();
   ABI_REQ(result && n > 0 && reps > 0, "bad argument");
   cudaEvent_t e0, e1;

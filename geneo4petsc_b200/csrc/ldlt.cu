@@ -14,7 +14,6 @@
 //   k_solve_ring<1 | 8 | 16>   ONE persistent cooperative launch per solve over a forest of factors; the factor tiles stream
 //                   through warp-private cp.async rings that run ahead of the arithmetic across items and level barriers
 //                   (HBM-bound by design); 8 / 16 right-hand sides use DMMA fragments
-//   k_solve_forest<2 | 4>      generic level-scheduled kernels for the other block widths
 #include "ldlt.hpp"
 
 #include <cooperative_groups.h>
@@ -33,6 +32,9 @@ constexpr int TS = 64;     // tile edge
 constexpr int KC = 16;     // K chunk per stage
 constexpr int SLD = 68;    // padded smem leading dimension (conflict-free 64-bit fragment loads)
 constexpr int GEMM_THREADS = 128;
+// cp.async pipeline depth of the DMMA tile kernels: 2 stages allow 5 CTAs per SM, 3 only 4 -- measured: 27.1 vs 24.6
+// TFLOP/s on the rank-128 update, occupancy beats depth
+constexpr int GEMM_STAGES = 2;
 
 __device__ __forceinline__ void dmma8x8x4(double& d0, double& d1, double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
@@ -40,7 +42,8 @@ __device__ __forceinline__ void dmma8x8x4(double& d0, double& d1, double a, doub
                : "d"(a), "d"(b));
 }
 
-constexpr int gemm_smem(int stages) { return stages * 2 * KC * SLD * 8; }  // bytes of dynamic shared memory per CTA
+constexpr int GEMM_SMEM = GEMM_STAGES * 2 * KC * SLD * 8;  // bytes of dynamic shared memory per CTA
+static_assert(GEMM_SMEM <= 48 * 1024, "the tile kernels launch without raising their dynamic shared memory limit");
 
 // 8-byte asynchronous copy global -> shared; srcBytes = 0 zero-fills (rows / columns outside the matrix)
 __device__ __forceinline__ void cp_async8(double* smem, const double* gmem, int srcBytes) {
@@ -56,7 +59,6 @@ __device__ __forceinline__ void cp_async_wait_g() { asm volatile("cp.async.wait_
 // fed while another CTA is in its prologue or read-modify-writing its C tile); one __syncthreads per K chunk.
 // The K dimension may come in TWO segments (A | A2)(B | B2)^T with their own leading dimensions (K2 = 0: one segment): the
 // rank-256 trailing update of a chain pair multiplies the panels of two consecutive fronts in one pass over the C tile.
-template <int GEMM_STAGES>
 __device__ void gemm_tile_nt(const double* __restrict__ A, int lda, int M, const double* __restrict__ B, int ldb,
                              int N, int K, double* __restrict__ C, int ldc, int mode, double* smem,
                              const double* __restrict__ A2 = nullptr, int lda2 = 0, const double* __restrict__ B2 = nullptr,
@@ -143,13 +145,12 @@ __device__ void gemm_tile_nt(const double* __restrict__ A, int lda, int M, const
     }
 }
 
-template <int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS) k_dgemm_nt(int M, int N, int K, const double* A, int lda,
                                                            const double* B, int ldb, double* C, int ldc, int mode) {
   extern __shared__ __align__(16) double gsm[];
   const int ti = blockIdx.x, tj = blockIdx.y;
-  gemm_tile_nt<STAGES>(A + ti * TS, lda, min(TS, M - ti * TS), B + tj * TS, ldb, min(TS, N - tj * TS), K,
-                       C + ti * TS + (size_t)tj * TS * ldc, ldc, mode, gsm);
+  gemm_tile_nt(A + ti * TS, lda, min(TS, M - ti * TS), B + tj * TS, ldb, min(TS, N - tj * TS), K,
+               C + ti * TS + (size_t)tj * TS * ldc, ldc, mode, gsm);
 }
 
 // =====================================================================================================================
@@ -312,7 +313,6 @@ __global__ void __launch_bounds__(256) k_copy_panel(const WorkItem* __restrict__
     if (c0 + c < k) dst[(size_t)c * m] = v[c];
 }
 
-template <int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS) k_panel(const WorkItem* __restrict__ items,
                                                         const FrontDev* __restrict__ fr, double* __restrict__ L,
                                                         const double* __restrict__ W) {
@@ -322,11 +322,10 @@ __global__ void __launch_bounds__(GEMM_THREADS) k_panel(const WorkItem* __restri
   const int m = F.h - F.k, k = F.k, h = F.ld;
   double* P = L + F.lOff;
   // L21[ti rows, tj cols] = W[ti rows, :] * Dinv[tj rows, :]^T   (Dinv symmetric)
-  gemm_tile_nt<STAGES>(W + F.wOff + it.a * TS, m, min(TS, m - it.a * TS), P + it.b * TS, h, min(TS, k - it.b * TS), k,
+  gemm_tile_nt(W + F.wOff + it.a * TS, m, min(TS, m - it.a * TS), P + it.b * TS, h, min(TS, k - it.b * TS), k,
                P + k + it.a * TS + (size_t)it.b * TS * h, h, 0, gsm);
 }
 
-template <int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS, 5) k_schur(const WorkItem* __restrict__ items,
                                                         const FrontDev* __restrict__ fr, const double* __restrict__ L,
                                                         const double* __restrict__ W, UArenas ua) {
@@ -338,13 +337,12 @@ __global__ void __launch_bounds__(GEMM_THREADS, 5) k_schur(const WorkItem* __res
   // tile: the rank-256 update of the next level covers everything from column k' on)
   const int ncols = F.pair == 1 ? min(m, fr[it.f + 1].k) : m;
   // U[ti, tj] -= L21[ti rows, :] * W[tj rows, :]^T   (lower triangle of tiles only)
-  gemm_tile_nt<STAGES>(L + F.lOff + k + it.a * TS, h, min(TS, m - it.a * TS), W + F.wOff + it.b * TS, m,
+  gemm_tile_nt(L + F.lOff + k + it.a * TS, h, min(TS, m - it.a * TS), W + F.wOff + it.b * TS, m,
                min(TS, ncols - it.b * TS), k, ua.a[F.uArena] + F.uOff + it.a * TS + (size_t)it.b * TS * F.uLd, F.uLd, 1, gsm);
 }
 
 // Second panel of a chain pair: U -= [L21_prev(rows below this panel's pivots) | L21] [W_prev(same rows) | W]^T, K = k_prev + k.
 // The first panel of the pair only updated the strip of U this panel assembled (its own k pivot columns).
-template <int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS, 5) k_schur2(const WorkItem* __restrict__ items, const FrontDev* __restrict__ fr,
                                                          const double* __restrict__ L, const double* __restrict__ Wcur,
                                                          const double* __restrict__ Wprev, UArenas ua) {
@@ -353,9 +351,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 5) k_schur2(const WorkItem* __re
   const FrontDev F = fr[it.f];
   const FrontDev Pf = fr[it.f - 1];
   const int m = F.h - F.k, k = F.k, pm = Pf.h - Pf.k;
-  gemm_tile_nt<STAGES>(L + Pf.lOff + Pf.k + k + it.a * TS, Pf.ld, min(TS, m - it.a * TS), Wprev + Pf.wOff + k + it.b * TS, pm,
-                       min(TS, m - it.b * TS), Pf.k, ua.a[F.uArena] + F.uOff + it.a * TS + (size_t)it.b * TS * F.uLd, F.uLd, 1, gsm,
-                       L + F.lOff + k + it.a * TS, F.ld, Wcur + F.wOff + it.b * TS, m, k);
+  gemm_tile_nt(L + Pf.lOff + Pf.k + k + it.a * TS, Pf.ld, min(TS, m - it.a * TS), Wprev + Pf.wOff + k + it.b * TS, pm,
+               min(TS, m - it.b * TS), Pf.k, ua.a[F.uArena] + F.uOff + it.a * TS + (size_t)it.b * TS * F.uLd, F.uLd, 1, gsm,
+               L + F.lOff + k + it.a * TS, F.ld, Wcur + F.wOff + it.b * TS, m, k);
 }
 
 // =====================================================================================================================
@@ -365,210 +363,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 5) k_schur2(const WorkItem* __re
 //                                are D^-1 (-> Y += ...), the rest are L21 (-> X[rows] -= ...): one uniform GEMV stream.
 //   backward:                    y1[c0:c1] -= L21[:, c0:c1]^T * y2
 //
-// A work item is (subdomain, front, row tile, 32-column chunk).  A warp streams its tile with 16-byte loads (2 rows per
-// lane; panels have an even leading dimension), 8..32 independent loads in flight per lane, so that a few warps per SM
-// already cover the HBM latency-bandwidth product.  The backward (transposed) product keeps one accumulator per column
-// and finishes with a 31-shuffle butterfly transpose-reduction instead of 32 separate warp reductions.
 // Levels are separated by grid-wide barriers instead of kernel launches: one launch and 2*levels barriers per solve.
 // =====================================================================================================================
-constexpr int SOLVE_COLS = 32;
-constexpr int FWD_ROWS = 64;
-constexpr int BWD_ROWS = 128;
-constexpr int SOLVE_THREADS = 512;
-
-__device__ __forceinline__ double2 ldg2(const double* p) { return __ldg(reinterpret_cast<const double2*>(p)); }
-__device__ __forceinline__ ForestItem load_item(const ForestItem* p) {
-  const int4* q = reinterpret_cast<const int4*>(p);
-  union { int4 v[3]; ForestItem it; } u;
-  u.v[0] = __ldg(q); u.v[1] = __ldg(q + 1); u.v[2] = __ldg(q + 2);
-  return u.it;
-}
 constexpr int MAX_SMEM_SUBS = 64;
-
-template <int NR>
-__device__ __forceinline__ void fwd_item(const ForestSub& S, const ForestItem& it, int part, double* __restrict__ X,
-                                         double* __restrict__ Y, int ldx, int lane) {
-  constexpr int FS = NR >= 4 ? 4 : 1;  // a block solve splits the 32 columns of an item into FS virtual items
-  constexpr int UN = NR == 1 ? 16 : 8; // independent 16-byte loads in flight per lane
-  const int k = it.k, h = it.h, ld = it.ld;
-  const int cs = part * (SOLVE_COLS / FS);
-  const int nc = min(SOLVE_COLS / FS, it.nc - cs);
-  if (nc <= 0) return;
-  const int r0 = it.r0 + 2 * lane;  // panel rows r0, r0+1 (even: 16-byte aligned)
-  const double* x1 = X + (size_t)(S.xoff + it.col0 + it.c0 + cs) * ldx;
-  const double* Lp = S.L + it.lOff + (size_t)cs * ld + (r0 < h ? 2 * lane : 0);
-  double xv = 0.;
-  if (NR == 1) xv = lane < nc ? x1[lane] : 0.;
-  // target rows of the two results: issued now so that they travel together with the factor loads
-  int row0 = -1, row1 = -1;
-  if (r0 >= k && r0 < h) row0 = S.rowIdx[it.rowOff + r0];
-  if (r0 + 1 >= k && r0 + 1 < h) row1 = S.rowIdx[it.rowOff + r0 + 1];
-  double a0[NR], a1[NR];
-#pragma unroll
-  for (int j = 0; j < NR; j++) a0[j] = a1[j] = 0.;
-  int c = 0;
-  for (; c + UN <= nc; c += UN) {
-    double2 v[UN];
-#pragma unroll
-    for (int u = 0; u < UN; u++) v[u] = ldg2(Lp + (size_t)(c + u) * ld);
-#pragma unroll
-    for (int u = 0; u < UN; u++) {
-      if (NR == 1) {
-        const double xc = __shfl_sync(0xffffffffu, xv, c + u);
-        a0[0] += v[u].x * xc;
-        a1[0] += v[u].y * xc;
-      } else {
-#pragma unroll
-        for (int j = 0; j < NR; j++) {
-          const double xc = x1[(size_t)(c + u) * ldx + j];
-          a0[j] += v[u].x * xc;
-          a1[j] += v[u].y * xc;
-        }
-      }
-    }
-  }
-  for (; c < nc; c++) {
-    const double2 v = ldg2(Lp + (size_t)c * ld);
-    if (NR == 1) {
-      const double xc = __shfl_sync(0xffffffffu, xv, c);
-      a0[0] += v.x * xc;
-      a1[0] += v.y * xc;
-    } else {
-#pragma unroll
-      for (int j = 0; j < NR; j++) {
-        const double xc = x1[(size_t)c * ldx + j];
-        a0[j] += v.x * xc;
-        a1[j] += v.y * xc;
-      }
-    }
-  }
-#pragma unroll
-  for (int e = 0; e < 2; e++) {
-    const int r = r0 + e;
-    if (r >= h) continue;
-    if (r < k) {  // D^-1 rows
-      double* dst = Y + (size_t)(S.xoff + it.col0 + r) * ldx;
-#pragma unroll
-      for (int j = 0; j < NR; j++) atomicAdd(dst + j, e ? a1[j] : a0[j]);
-    } else {      // L21 rows
-      double* dst = X + (size_t)(S.xoff + (e ? row1 : row0)) * ldx;
-#pragma unroll
-      for (int j = 0; j < NR; j++) atomicAdd(dst + j, -(e ? a1[j] : a0[j]));
-    }
-  }
-}
-
-// transposed product: one accumulator per (column, rhs) pair; PC = 16 / NR (NR <= 8) columns per pass keep the
-// accumulators + the loads in flight inside the register budget
-template <int NR>
-__device__ __forceinline__ void bwd_item(const ForestSub& S, const ForestItem& it, int pass, double* __restrict__ Y, int ldx, int lane) {
-  constexpr int NA = NR == 1 ? 16 : 32;  // accumulators per lane
-  constexpr int CP = NA / NR;            // columns per pass
-  const int k = it.k, h = it.h, ld = it.ld;
-  const int cp = pass * CP;  // the 32 columns of an item are split into 32/CP independent passes (virtual items)
-  if (cp >= it.nc) return;
-  const int rbase = it.r0 + 2 * lane;  // even panel row; rows < k are masked out through y = 0
-  double y0[2][NR], y1[2][NR];
-  const double* Lt[2];
-#pragma unroll
-  for (int t = 0; t < 2; t++) {
-    const int r = rbase + t * 64;
-    const bool ok0 = r >= k && r < h, ok1 = r + 1 >= k && r + 1 < h;
-    const int row0 = ok0 ? S.rowIdx[it.rowOff + r] : 0, row1 = ok1 ? S.rowIdx[it.rowOff + r + 1] : 0;
-#pragma unroll
-    for (int j = 0; j < NR; j++) {
-      y0[t][j] = ok0 ? Y[(size_t)(S.xoff + row0) * ldx + j] : 0.;
-      y1[t][j] = ok1 ? Y[(size_t)(S.xoff + row1) * ldx + j] : 0.;
-    }
-    Lt[t] = S.L + it.lOff + (size_t)cp * ld + (r < h ? 2 * lane + t * 64 : 0);
-  }
-  double acc[NA];
-#pragma unroll
-  for (int q = 0; q < NA; q++) acc[q] = 0.;
-#pragma unroll
-  for (int t = 0; t < 2; t++) {
-#pragma unroll
-    for (int cc = 0; cc < CP; cc++) {
-      if (cp + cc < it.nc) {  // warp-uniform
-        const double2 v = ldg2(Lt[t] + (size_t)cc * ld);
-#pragma unroll
-        for (int j = 0; j < NR; j++) acc[cc * NR + j] += v.x * y0[t][j] + v.y * y1[t][j];
-      }
-    }
-  }
-  // butterfly transpose-reduction: NA values over 32 lanes; lane q (mod NA) ends up with the warp-wide sum of acc[q]
-  if (NA == 16) {  // first fold the two half-warps onto each other
-#pragma unroll
-    for (int q = 0; q < 16; q++) acc[q] += __shfl_xor_sync(0xffffffffu, acc[q], 16);
-  }
-#pragma unroll
-  for (int off = (NA == 16 ? 8 : 16); off >= 1; off >>= 1) {
-    const bool upper = (lane & off) != 0;
-#pragma unroll
-    for (int i = 0; i < off; i++) {
-      const double send = upper ? acc[i] : acc[i + off];
-      const double keep = upper ? acc[i + off] : acc[i];
-      acc[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
-    }
-  }
-  const int q = NA == 16 ? (lane & 15) : lane;
-  const int cc = q / NR, j = q % NR;
-  if ((NA == 32 || lane < 16) && cp + cc < it.nc)
-    atomicAdd(&Y[(size_t)(S.xoff + it.col0 + it.c0 + cp + cc) * ldx + j], -acc[0]);
-}
-
-template <int NR>
-__global__ void __launch_bounds__(SOLVE_THREADS, 1)
-k_solve_forest(const ForestSub* __restrict__ subs, int nsubs, const ForestItem* __restrict__ items, const int64_t* __restrict__ ranges,
-               int nlev, int64_t ntot, double* __restrict__ X, double* __restrict__ Y, int ldx) {
-  cg::grid_group grid = cg::this_grid();
-  __shared__ ForestSub sSubs[MAX_SMEM_SUBS];
-  for (int t = threadIdx.x; t < min(nsubs, MAX_SMEM_SUBS); t += blockDim.x) sSubs[t] = subs[t];
-  const bool inSmem = nsubs <= MAX_SMEM_SUBS;
-  const int lane = threadIdx.x & 31;
-  const int64_t gw = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  // Y = 0 (the forward sweep accumulates D^-1 x into it); visible to everyone after the first barrier
-  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < ntot * NR; t += (int64_t)gridDim.x * blockDim.x)
-    Y[(t / NR) * ldx + (t % NR)] = 0.;
-  grid.sync();
-  const int64_t* fwdOff = ranges;
-  const int64_t* fwdCnt = ranges + nlev;
-  const int64_t* bwdOff = ranges + 2 * nlev;
-  const int64_t* bwdCnt = ranges + 3 * nlev;
-  constexpr int FS = NR >= 4 ? 4 : 1;
-  constexpr int BP = 32 / ((NR == 1 ? 16 : 32) / NR);  // backward passes per item
-  for (int l = 0; l < nlev; l++) {
-    const int64_t off = fwdOff[l], cnt = fwdCnt[l] * FS;
-    int64_t i = gw;
-    ForestItem cur;
-    if (i < cnt) cur = load_item(items + off + i / FS);
-    while (i < cnt) {
-      const int64_t in = i + nw;
-      ForestItem nxt = cur;
-      if (in < cnt) nxt = load_item(items + off + in / FS);  // the next item's record travels while this one streams
-      fwd_item<NR>(inSmem ? sSubs[cur.sub] : subs[cur.sub], cur, (int)(i % FS), X, Y, ldx, lane);
-      cur = nxt;
-      i = in;
-    }
-    grid.sync();
-  }
-  for (int l = nlev - 1; l >= 0; l--) {
-    const int64_t off = bwdOff[l], cnt = bwdCnt[l] * BP;
-    int64_t i = gw;
-    ForestItem cur;
-    if (i < cnt) cur = load_item(items + off + i / BP);
-    while (i < cnt) {
-      const int64_t in = i + nw;
-      ForestItem nxt = cur;
-      if (in < cnt) nxt = load_item(items + off + in / BP);
-      bwd_item<NR>(inSmem ? sSubs[cur.sub] : subs[cur.sub], cur, (int)(i % BP), Y, ldx, lane);
-      cur = nxt;
-      i = in;
-    }
-    if (l > 0) grid.sync();
-  }
-}
 
 // ---------------------------------------------------------------------------------------------------------------------
 // Ring-buffered streaming solve: NR = 1 (the preconditioner application) and NR = 8 (block solves of the eigen-solver
@@ -602,16 +399,13 @@ template <int W, int STAGES, int CSTRIDE, int BC> struct RingCfgT {
   static constexpr int WARP_BYTES = STAGES * STAGE + RING_RS * 48;
   static constexpr int SMEM = W * WARP_BYTES;
 };
-template <int NR, int VAR> struct RingCfg;   // VAR: tuning variant (GENEO_RING_VAR, default 0)
-template <> struct RingCfg<1, 0> : RingCfgT<16, 3, 64, 16> {};  // 16 warps x 3 stages: 128 KB in flight per SM, <= 128 registers
-template <> struct RingCfg<1, 1> : RingCfgT<12, 4, 64, 16> {};  // 12 warps x 4 stages: 144 KB in flight per SM, <= 168 registers
-template <> struct RingCfg<8, 0> : RingCfgT<12, 4, 68, 32> {};  // 12 warps x 4 stages: 144 KB in flight per SM, <= 168 registers
-template <> struct RingCfg<8, 1> : RingCfgT<12, 4, 68, 32> {};
+template <int NR> struct RingCfg;
+template <> struct RingCfg<1> : RingCfgT<16, 3, 64, 16> {};  // 16 warps x 3 stages: 128 KB in flight per SM, <= 128 registers
+template <> struct RingCfg<8> : RingCfgT<12, 4, 68, 32> {};  // 12 warps x 4 stages: 144 KB in flight per SM, <= 168 registers
 // NR = 16 walks the item lists of NR = 8 with two DMMAs per L fragment.  8 warps = 2 per SM sub-partition: the register file
 // of a sub-partition (16 K registers) then allows 255 registers per thread (10 or 12 warps put 3 on one sub-partition: 168);
 // 6 stages keep 160 KB in flight per SM.
-template <> struct RingCfg<16, 0> : RingCfgT<8, 6, 68, 32> {};
-template <> struct RingCfg<16, 1> : RingCfgT<8, 6, 68, 32> {};
+template <> struct RingCfg<16> : RingCfgT<8, 6, 68, 32> {};
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
@@ -634,16 +428,16 @@ __device__ __forceinline__ RingRec load_ring_item(const RingItem* p) {
 }
 __device__ __forceinline__ int64_t rec_i64(int lo, int hi) { return (int64_t)(((unsigned long long)(unsigned)hi << 32) | (unsigned)lo); }
 
-template <int NR, int VAR>
-__global__ void __launch_bounds__(RingCfg<NR, VAR>::WARPS * 32, 1)
+template <int NR>
+__global__ void __launch_bounds__(RingCfg<NR>::WARPS * 32, 1)
 k_solve_ring(const ForestSub* __restrict__ subs, int nsubs, const RingItem* __restrict__ items,
              const int64_t* __restrict__ ranges, int nlev, int64_t ntot, double* __restrict__ X, double* __restrict__ Y,
-             int ldx, long long* __restrict__ tstamp, int flags) {
-  constexpr int CS = RingCfg<NR, VAR>::CS;
-  constexpr int RING_S = RingCfg<NR, VAR>::S;
+             int ldx, long long* __restrict__ tstamp) {
+  constexpr int CS = RingCfg<NR>::CS;
+  constexpr int RING_S = RingCfg<NR>::S;
   constexpr int TILE_BYTES = RING_CH * CS * 8;
-  constexpr int STAGE = RingCfg<NR, VAR>::STAGE;
-  constexpr int BWD_COLS = RingCfg<NR, VAR>::BWD_COLS;
+  constexpr int STAGE = RingCfg<NR>::STAGE;
+  constexpr int BWD_COLS = RingCfg<NR>::BWD_COLS;
   cg::grid_group grid = cg::this_grid();
   extern __shared__ __align__(16) unsigned char ringmem[];
   __shared__ ForestSub sSubs[MAX_SMEM_SUBS];
@@ -660,13 +454,13 @@ k_solve_ring(const ForestSub* __restrict__ subs, int nsubs, const RingItem* __re
       sCnt[p] = (int)ranges[(b ? 3 * nlev : nlev) + l];
     }
   if (NR > 1)  // fragments read whole stages: never let a NaN pattern of uninitialised shared memory into a product
-    for (int t = threadIdx.x; t < RingCfg<NR, VAR>::SMEM / 16; t += blockDim.x) reinterpret_cast<int4*>(ringmem)[t] = make_int4(0, 0, 0, 0);
+    for (int t = threadIdx.x; t < RingCfg<NR>::SMEM / 16; t += blockDim.x) reinterpret_cast<int4*>(ringmem)[t] = make_int4(0, 0, 0, 0);
   const bool inSmem = nsubs <= MAX_SMEM_SUBS;
   const int lane = threadIdx.x & 31;
-  unsigned char* wmem = ringmem + (threadIdx.x >> 5) * RingCfg<NR, VAR>::WARP_BYTES;
+  unsigned char* wmem = ringmem + (threadIdx.x >> 5) * RingCfg<NR>::WARP_BYTES;
   int4* recRing = reinterpret_cast<int4*>(wmem + RING_S * STAGE);
   // consecutive items of a phase go to different SMs: a level with few items still uses every SM's LSU / L1 / RED path
-  const int64_t gw = (flags & 1) ? ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5 : (int64_t)(threadIdx.x >> 5) * gridDim.x + blockIdx.x;
+  const int64_t gw = (int64_t)(threadIdx.x >> 5) * gridDim.x + blockIdx.x;
   const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < ntot * NR; t += (int64_t)gridDim.x * blockDim.x)
     Y[(t / NR) * ldx + (t % NR)] = 0.;
@@ -804,7 +598,7 @@ k_solve_ring(const ForestSub* __restrict__ subs, int nsubs, const RingItem* __re
               const int2 ri = *reinterpret_cast<const int2*>(st + TILE_BYTES + 8 * lane);
               row0 = ri.x; row1 = ri.y;
             }
-            if (q == Q - 1 && i + nw < cnt && !(flags & 2)) {  // the next item's record has been handed over by now (RING_S >= 2)
+            if (q == Q - 1 && i + nw < cnt) {  // the next item's record has been handed over by now (RING_S >= 2)
               __syncwarp();
               const int4* r2 = recRing + (cm & (RING_RS - 1)) * 3;
               const int4 b2 = r2[1], c2 = r2[2];
@@ -1020,7 +814,7 @@ k_solve_ring(const ForestSub* __restrict__ subs, int nsubs, const RingItem* __re
         }
       }
     }
-    if (!(flags & 4)) top_up();  // idle warps keep scanning ahead / prefetching here, off everybody's critical path
+    top_up();  // idle warps keep scanning ahead / prefetching here, off everybody's critical path
     if (p + 1 < nph) {
       grid.sync();
       if (tstamp && blockIdx.x == 0 && threadIdx.x == 0) tstamp[p + 1] = gtimer();
@@ -1032,32 +826,10 @@ k_solve_ring(const ForestSub* __restrict__ subs, int nsubs, const RingItem* __re
 
 }  // namespace
 
-static int gemm_stages() {  // cp.async pipeline depth of the DMMA tile kernels: 3 (4 CTAs per SM) or 2 (5 CTAs per SM)
-  static const int v = [] {
-    const char* e = getenv("GENEO_GEMM_STAGES");
-    const int st = (e && atoi(e) == 3) ? 3 : 2;  // measured: 27.1 vs 24.6 TFLOP/s on the rank-128 update, occupancy beats depth
-    const int sm = gemm_smem(st);
-    if (st == 2) {
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_dgemm_nt<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_panel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_schur<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_schur2<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-    } else {
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_dgemm_nt<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_panel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_schur<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-      CUDA_CHECK(cudaFuncSetAttribute((const void*)k_schur2<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));
-    }
-    return st;
-  }();
-  return v;
-}
-
 void dgemm_nt_device(int M, int N, int K, const double* A, int lda, const double* B, int ldb, double* C, int ldc,
                      int mode, cudaStream_t st) {
   dim3 grid((M + TS - 1) / TS, (N + TS - 1) / TS);
-  if (gemm_stages() == 2) k_dgemm_nt<2><<<GENEO_TICK(grid), GEMM_THREADS, gemm_smem(2), st>>>(M, N, K, A, lda, B, ldb, C, ldc, mode);
-  else k_dgemm_nt<3><<<GENEO_TICK(grid), GEMM_THREADS, gemm_smem(3), st>>>(M, N, K, A, lda, B, ldb, C, ldc, mode);
+  k_dgemm_nt<<<GENEO_TICK(grid), GEMM_THREADS, GEMM_SMEM, st>>>(M, N, K, A, lda, B, ldb, C, ldc, mode);
   CUDA_CHECK(cudaGetLastError());
 }
 
@@ -1203,7 +975,7 @@ void factor_prepare(FactorJob& J) {
   CUDA_CHECK(cudaGetLastError());
 }
 
-void factor_level(FactorJob& J, int l, int gst) {
+void factor_level(FactorJob& J, int l) {
   const LdltPlan& P = J.F->plan();
   LdltWorkspace& ws = *J.ws;
   cudaStream_t st = J.st;
@@ -1224,30 +996,23 @@ void factor_level(FactorJob& J, int l, int gst) {
     k_diag_invert<32, 8><<<GENEO_TICK(P.diagSmallItems[l].cnt), 64, 0, st>>>(items + P.diagSmallItems[l].off, P.dFronts.p, Lp, pivTol, ws.counters.p);
   if (P.copyItems[l].cnt)
     k_copy_panel<<<GENEO_TICK(P.copyItems[l].cnt), 256, 0, st>>>(items + P.copyItems[l].off, P.dFronts.p, Lp, Wcur);
-  if (P.panelItems[l].cnt) {
-    if (gst == 2) k_panel<2><<<GENEO_TICK(P.panelItems[l].cnt), GEMM_THREADS, gemm_smem(2), st>>>(items + P.panelItems[l].off, P.dFronts.p, Lp, Wcur);
-    else k_panel<3><<<GENEO_TICK(P.panelItems[l].cnt), GEMM_THREADS, gemm_smem(3), st>>>(items + P.panelItems[l].off, P.dFronts.p, Lp, Wcur);
-  }
-  if (P.schurItems[l].cnt) {
-    if (gst == 2) k_schur<2><<<GENEO_TICK(P.schurItems[l].cnt), GEMM_THREADS, gemm_smem(2), st>>>(items + P.schurItems[l].off, P.dFronts.p, Lp, Wcur, ua);
-    else k_schur<3><<<GENEO_TICK(P.schurItems[l].cnt), GEMM_THREADS, gemm_smem(3), st>>>(items + P.schurItems[l].off, P.dFronts.p, Lp, Wcur, ua);
-  }
-  if (P.schur2Items[l].cnt) {
-    if (gst == 2) k_schur2<2><<<GENEO_TICK(P.schur2Items[l].cnt), GEMM_THREADS, gemm_smem(2), st>>>(items + P.schur2Items[l].off, P.dFronts.p, Lp, Wcur, Wprev, ua);
-    else k_schur2<3><<<GENEO_TICK(P.schur2Items[l].cnt), GEMM_THREADS, gemm_smem(3), st>>>(items + P.schur2Items[l].off, P.dFronts.p, Lp, Wcur, Wprev, ua);
-  }
+  if (P.panelItems[l].cnt)
+    k_panel<<<GENEO_TICK(P.panelItems[l].cnt), GEMM_THREADS, GEMM_SMEM, st>>>(items + P.panelItems[l].off, P.dFronts.p, Lp, Wcur);
+  if (P.schurItems[l].cnt)
+    k_schur<<<GENEO_TICK(P.schurItems[l].cnt), GEMM_THREADS, GEMM_SMEM, st>>>(items + P.schurItems[l].off, P.dFronts.p, Lp, Wcur, ua);
+  if (P.schur2Items[l].cnt)
+    k_schur2<<<GENEO_TICK(P.schur2Items[l].cnt), GEMM_THREADS, GEMM_SMEM, st>>>(items + P.schur2Items[l].off, P.dFronts.p, Lp, Wcur, Wprev, ua);
   CUDA_CHECK(cudaGetLastError());
 }
 }  // namespace
 
 void factorize_enqueue(std::vector<FactorJob>& jobs) {
-  const int gst = gemm_stages();
   int gmax = 0;
   for (auto& J : jobs) { factor_prepare(J); gmax = std::max(gmax, J.F->plan().sym.nlevels); }
   for (int g = 0; g < gmax; g++)
     for (auto& J : jobs) {
       const int l = g - (gmax - J.F->plan().sym.nlevels);  // roots aligned
-      if (l >= 0) factor_level(J, l, gst);
+      if (l >= 0) factor_level(J, l);
     }
   for (auto& J : jobs)
     if (J.hostCounters) CUDA_CHECK(cudaMemcpyAsync(J.hostCounters, J.ws->counters.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, J.st));
@@ -1268,22 +1033,13 @@ FactorStats LdltFactor::factorize(const double* dVals, double pivTol, LdltWorksp
   return stats;
 }
 
-static int ring_var() {  // tuning variant of the ring kernels: read when a forest is built, fixed for that forest
-  const char* e = getenv("GENEO_RING_VAR");
-  return e ? (atoi(e) != 0 ? 1 : 0) : 0;
-}
 struct RingLaunch { const void* fn; int warps, smem, bwdCols; };
-static RingLaunch ring_launch(int which, int v) {
-  if (which == 0) {
-    if (v == 0) return RingLaunch{(const void*)k_solve_ring<1, 0>, RingCfg<1, 0>::WARPS, RingCfg<1, 0>::SMEM, RingCfg<1, 0>::BWD_COLS};
-    return RingLaunch{(const void*)k_solve_ring<1, 1>, RingCfg<1, 1>::WARPS, RingCfg<1, 1>::SMEM, RingCfg<1, 1>::BWD_COLS};
-  }
-  if (which == 2) {  // NR = 16 (shares the item lists of NR = 8)
-    if (v == 0) return RingLaunch{(const void*)k_solve_ring<16, 0>, RingCfg<16, 0>::WARPS, RingCfg<16, 0>::SMEM, RingCfg<16, 0>::BWD_COLS};
-    return RingLaunch{(const void*)k_solve_ring<16, 1>, RingCfg<16, 1>::WARPS, RingCfg<16, 1>::SMEM, RingCfg<16, 1>::BWD_COLS};
-  }
-  if (v == 0) return RingLaunch{(const void*)k_solve_ring<8, 0>, RingCfg<8, 0>::WARPS, RingCfg<8, 0>::SMEM, RingCfg<8, 0>::BWD_COLS};
-  return RingLaunch{(const void*)k_solve_ring<8, 1>, RingCfg<8, 1>::WARPS, RingCfg<8, 1>::SMEM, RingCfg<8, 1>::BWD_COLS};
+static RingLaunch ring_launch(int which) {  // which = 0: NR = 1, 1: NR = 8, 2: NR = 16 (shares the item lists of NR = 8)
+  static const RingLaunch table[3] = {
+      {(const void*)k_solve_ring<1>, RingCfg<1>::WARPS, RingCfg<1>::SMEM, RingCfg<1>::BWD_COLS},
+      {(const void*)k_solve_ring<8>, RingCfg<8>::WARPS, RingCfg<8>::SMEM, RingCfg<8>::BWD_COLS},
+      {(const void*)k_solve_ring<16>, RingCfg<16>::WARPS, RingCfg<16>::SMEM, RingCfg<16>::BWD_COLS}};
+  return table[which];
 }
 
 // =====================================================================================================================
@@ -1296,7 +1052,7 @@ void SolveForest::build(const std::vector<const LdltPlan*>& plans, const std::ve
   nlev = 0;
   ntot = 0;
   for (int s = 0; s < ns; s++) { nlev = std::max(nlev, plans[s]->sym.nlevels); ntot = std::max<int64_t>(ntot, xoff[s] + plans[s]->sym.n); }
-  genericBuilt = ringBuilt[0] = ringBuilt[1] = false;
+  ringBuilt[0] = ringBuilt[1] = false;
   hSubs.assign(ns, ForestSub{nullptr, nullptr, nullptr, 0});
   for (int s = 0; s < ns; s++) { hSubs[s].fronts = plans[s]->dFronts.p; hSubs[s].rowIdx = plans[s]->dRowIdx.p; hSubs[s].xoff = xoff[s]; }
   dSubs.alloc(ns);
@@ -1304,81 +1060,18 @@ void SolveForest::build(const std::vector<const LdltPlan*>& plans, const std::ve
   int dev = 0, nsm = 0;
   CUDA_CHECK(cudaGetDevice(&dev));
   CUDA_CHECK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev));
-  const void* fns[4] = {(const void*)k_solve_forest<1>, (const void*)k_solve_forest<2>, (const void*)k_solve_forest<4>, (const void*)k_solve_forest<8>};
-  for (int q = 0; q < 4; q++) {
+  for (int which = 0; which < 3; which++) {
+    const RingLaunch rl = ring_launch(which);
     int nb = 0;
-    CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fns[q], SOLVE_THREADS, 0));
-    gridBlocks[q] = std::max(1, nb) * nsm;
-  }
-  {
-    int nb = 0;
-    ringVar = ring_var();
-    for (int which = 0; which < 3; which++) {
-      const RingLaunch rl = ring_launch(which, ringVar);
-      CUDA_CHECK(cudaFuncSetAttribute(rl.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, rl.smem));
-      CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, rl.fn, rl.warps * 32, rl.smem));
-      if (which < 2) ringGrid[which] = std::max(1, nb) * nsm;
-      else ringGrid[1] = std::min(ringGrid[1], std::max(1, nb) * nsm);  // NR = 16 walks the NR = 8 lists on the SAME cooperative grid:
-                                                                          // it must fit both kernels (the warp -> item mapping is
-                                                                          // computed in the kernel from its own block size)
-    }
+    CUDA_CHECK(cudaFuncSetAttribute(rl.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, rl.smem));
+    CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, rl.fn, rl.warps * 32, rl.smem));
+    if (which < 2) ringGrid[which] = std::max(1, nb) * nsm;
+    else ringGrid[1] = std::min(ringGrid[1], std::max(1, nb) * nsm);  // NR = 16 walks the NR = 8 lists on the SAME cooperative grid:
+                                                                        // it must fit both kernels (the warp -> item mapping is
+                                                                        // computed in the kernel from its own block size)
   }
 }
 
-void SolveForest::build_generic() const {
-  HostProfScope hp("forest build (generic)");
-  const int ns = (int)plans_.size();
-  const std::vector<const LdltPlan*>& plans = plans_;
-  std::vector<ForestItem> items;
-  std::vector<int64_t> ranges(4 * (size_t)nlev, 0);
-  auto by_size = [](const ForestItem& a, const ForestItem& b) {  // big tiles first: the tail of a level is made of small ones
-    const int64_t sa = (int64_t)std::min(a.h - a.r0, BWD_ROWS) * a.nc, sb = (int64_t)std::min(b.h - b.r0, BWD_ROWS) * b.nc;
-    return sa > sb;
-  };
-  for (int l = 0; l < nlev; l++) {  // forward + diagonal: every row of the panel
-    ranges[l] = (int64_t)items.size();
-    for (int s = 0; s < ns; s++) {
-      const Symbolic& S = plans[s]->sym;
-      if (l >= S.nlevels) continue;
-      for (int t = S.levelPtr[l]; t < S.levelPtr[l + 1]; t++) {
-        const Front& F = S.fronts[S.levelFronts[t]];
-        for (int rb = 0; rb * FWD_ROWS < F.h; rb++)
-          for (int c0 = 0; c0 < F.k; c0 += SOLVE_COLS)
-            items.push_back(ForestItem{F.lOff + (int64_t)c0 * F.ld + rb * FWD_ROWS, F.rowOff, s, F.ld, F.h, F.k, c0,
-                                       std::min(SOLVE_COLS, F.k - c0), rb * FWD_ROWS, F.col0});
-      }
-    }
-    ranges[nlev + l] = (int64_t)items.size() - ranges[l];
-    std::stable_sort(items.begin() + ranges[l], items.end(), by_size);
-  }
-  for (int l = 0; l < nlev; l++) {  // backward: the L21 rows, tiles start at the even row k & ~1
-    ranges[2 * nlev + l] = (int64_t)items.size();
-    for (int s = 0; s < ns; s++) {
-      const Symbolic& S = plans[s]->sym;
-      if (l >= S.nlevels) continue;
-      for (int t = S.levelPtr[l]; t < S.levelPtr[l + 1]; t++) {
-        const Front& F = S.fronts[S.levelFronts[t]];
-        if (F.m() == 0) continue;
-        const int rstart = F.k & ~1;
-        for (int r0 = rstart; r0 < F.h; r0 += BWD_ROWS)
-          for (int c0 = 0; c0 < F.k; c0 += SOLVE_COLS)
-            items.push_back(ForestItem{F.lOff + (int64_t)c0 * F.ld + r0, F.rowOff, s, F.ld, F.h, F.k, c0,
-                                       std::min(SOLVE_COLS, F.k - c0), r0, F.col0});
-      }
-    }
-    ranges[3 * nlev + l] = (int64_t)items.size() - ranges[2 * nlev + l];
-    std::stable_sort(items.begin() + ranges[2 * nlev + l], items.end(), by_size);
-  }
-  dItems.upload(items);
-  dRanges.upload(ranges);
-  CUDA_CHECK(::geneo::sync_stream(0));
-  genericBuilt = true;
-}
-
-static int ring8_min_cspan() {
-  static const int v = [] { const char* e = getenv("GENEO_RING8_CSPAN"); const int c = e ? atoi(e) : 32; return c >= 128 ? 128 : c >= 64 ? 64 : 32; }();
-  return v;
-}
 // Item lists of the ring kernel.  Per level the host picks the span of an item from the amount of work in the level: a
 // level with many tiles per warp gets wide (forward: up to all 128 columns of a panel) / tall (backward: up to 512 rows)
 // items -- fewer records, x / y fetches and atomics per byte --, a level near the root gets the finest tiles so that every
@@ -1386,8 +1079,8 @@ static int ring8_min_cspan() {
 void SolveForest::build_ring(int which) const {
   HostProfScope hp("forest build (ring)");
   const int ns = (int)plans_.size();
-  const int warps = ring_launch(which, ringVar).warps;
-  const int RING_BWD_COLS = ring_launch(which, ringVar).bwdCols;
+  const int warps = ring_launch(which).warps;
+  const int RING_BWD_COLS = ring_launch(which).bwdCols;
   const int64_t nw = (int64_t)ringGrid[which] * warps;
   std::vector<RingItem> items;
   std::vector<int64_t> ranges(4 * (size_t)nlev, 0);
@@ -1409,11 +1102,8 @@ void SolveForest::build_ring(int which) const {
         bytes += 8. * F.h * F.k;
       }
     }
-    int cspan = 32 * pow2_floor(tiles / (4 * nw), 1, 4);
-    // (experiment hook GENEO_RING8_CSPAN: a wider minimum span for the block solves quarters their FP64 atomics per byte --
-    //  measured on 8 x 100^3: 3.25 s of eigen-solves with 32, 3.30 s with 64, 3.48 s with 128: not atomic-bound, the finest
-    //  tiles stay the default)
-    if (which >= 1) cspan = std::max(cspan, ring8_min_cspan());
+    // 32 is the floor for the block solves too: wider floors measured slower (8 x 100^3 eigen-solves: 3.25 / 3.30 / 3.48 s at 32 / 64 / 128)
+    const int cspan = 32 * pow2_floor(tiles / (4 * nw), 1, 4);
     ranges[l] = (int64_t)items.size();
     for (int s = 0; s < ns; s++) {
       const Symbolic& S = plans_[s]->sym;
@@ -1470,11 +1160,6 @@ void SolveForest::build_ring(int which) const {
   ringBuilt[which] = true;
 }
 
-static int ring_flags() {  // experiment switches of the ring kernel (GENEO_RING_FLAGS)
-  const char* e = getenv("GENEO_RING_FLAGS");
-  return e ? atoi(e) : 0;
-}
-
 void SolveForest::set_factors(const std::vector<const double*>& L, cudaStream_t st) {
   GENEO_CHECK(L.size() == hSubs.size(), "forest: wrong number of factors");
   for (size_t s = 0; s < L.size(); s++) hSubs[s].L = L[s];
@@ -1483,48 +1168,23 @@ void SolveForest::set_factors(const std::vector<const double*>& L, cudaStream_t 
 }
 
 void SolveForest::solve(double* X, double* Y, int ldx, int j0, int nr, cudaStream_t st) const {
+  GENEO_CHECK((nr == 1 && ldx == 1) || nr == 8 || nr == 16, "forest solve: nr must be 1 (with ldx = 1), 8 or 16");
   double* Xp = X + j0;
   double* Yp = Y + j0;
   const ForestSub* subs = dSubs.p;
   int nsubs = (int)hSubs.size();
-  const ForestItem* items = dItems.p;
-  const int64_t* ranges = dRanges.p;
   int nl = nlev;
   int64_t nt = ntot;
-  if (((nr == 1 && ldx == 1) || nr == 8 || nr == 16) && !getenv("GENEO_SOLVE_GENERIC")) {
-    const int which = nr == 1 ? 0 : 1;
-    if (!ringBuilt[which]) build_ring(which);
-    const RingItem* ritems = dRing[which].p;
-    const int64_t* rranges = dRingRanges[which].p;
-    long long* ts = nullptr;
-    int flags = ring_flags();
-    void* a1[] = {(void*)&subs, (void*)&nsubs, (void*)&ritems, (void*)&rranges, (void*)&nl, (void*)&nt, (void*)&Xp, (void*)&Yp,
-                  (void*)&ldx, (void*)&ts, (void*)&flags};
-    (void)GENEO_TICK(0);
-    const RingLaunch rl = ring_launch(nr == 16 ? 2 : which, ringVar);
-    CUDA_CHECK(cudaLaunchCooperativeKernel(rl.fn, dim3(ringGrid[which]), dim3(rl.warps * 32), a1, rl.smem, st));
-    return;
-  }
-  if (nr == 16) {  // (debug path GENEO_SOLVE_GENERIC: the generic kernels stop at 8 right-hand sides)
-    solve(X, Y, ldx, j0, 8, st);
-    solve(X, Y, ldx, j0 + 8, 8, st);
-    return;
-  }
-  if (!genericBuilt) build_generic();
-  items = dItems.p;
-  ranges = dRanges.p;
-  void* args[] = {(void*)&subs, (void*)&nsubs, (void*)&items, (void*)&ranges, (void*)&nl, (void*)&nt, (void*)&Xp, (void*)&Yp, (void*)&ldx};
-  const void* fn = nullptr;
-  int q = 0;
-  switch (nr) {
-    case 1: fn = (const void*)k_solve_forest<1>; q = 0; break;
-    case 2: fn = (const void*)k_solve_forest<2>; q = 1; break;
-    case 4: fn = (const void*)k_solve_forest<4>; q = 2; break;
-    case 8: fn = (const void*)k_solve_forest<8>; q = 3; break;
-    default: GENEO_CHECK(false, "nrhs chunk must be 1, 2, 4, 8 or 16");
-  }
+  const int which = nr == 1 ? 0 : 1;
+  if (!ringBuilt[which]) build_ring(which);
+  const RingItem* ritems = dRing[which].p;
+  const int64_t* rranges = dRingRanges[which].p;
+  long long* ts = nullptr;
+  void* a1[] = {(void*)&subs, (void*)&nsubs, (void*)&ritems, (void*)&rranges, (void*)&nl, (void*)&nt, (void*)&Xp, (void*)&Yp,
+                (void*)&ldx, (void*)&ts};
   (void)GENEO_TICK(0);
-  CUDA_CHECK(cudaLaunchCooperativeKernel(fn, dim3(gridBlocks[q]), dim3(SOLVE_THREADS), args, 0, st));
+  const RingLaunch rl = ring_launch(nr == 16 ? 2 : which);
+  CUDA_CHECK(cudaLaunchCooperativeKernel(rl.fn, dim3(ringGrid[which]), dim3(rl.warps * 32), a1, rl.smem, st));
 }
 
 void SolveForest::solve_profile(double* X, double* Y, int nr, std::vector<double>& us, std::vector<double>& bytes,
@@ -1541,11 +1201,10 @@ void SolveForest::solve_profile(double* X, double* Y, int nr, std::vector<double
   int ldx = nr;
   DevBuf<long long> dts((size_t)2 * nlev + 1);
   long long* ts = dts.p;
-  int flags = ring_flags();
   void* a1[] = {(void*)&subs, (void*)&nsubs, (void*)&ritems, (void*)&rranges, (void*)&nl, (void*)&nt, (void*)&X, (void*)&Y,
-                (void*)&ldx, (void*)&ts, (void*)&flags};
+                (void*)&ldx, (void*)&ts};
   (void)GENEO_TICK(0);
-  const RingLaunch rl = ring_launch(which, ringVar);
+  const RingLaunch rl = ring_launch(which);
   CUDA_CHECK(cudaLaunchCooperativeKernel(rl.fn, dim3(ringGrid[which]), dim3(rl.warps * 32), a1, rl.smem, 0));
   CUDA_CHECK(::geneo::sync_stream(0));
   std::vector<long long> h = dts.to_host();

@@ -52,9 +52,6 @@ class LdltPlan {
 
 // ---- level-scheduled solves over a forest of factors (one persistent cooperative kernel) -----------------------------
 struct ForestSub { const double* L; const FrontDev* fronts; const int* rowIdx; int64_t xoff; };
-// self-contained work item (48 bytes, three 16-byte loads): nothing but the subdomain's base pointers (kept in shared
-// memory) stands between reading the item and issuing the factor loads
-struct ForestItem { int64_t lOff, rowOff; int sub, ld, h, k; int c0, nc, r0, col0; };
 // item of the ring-buffered NR = 1 kernel (48 bytes): lOff / rowOff point at the tile origin (row r0, column c0) of the
 // panel and at rowIdx[r0]; nrows x nc is the extent of the item; the first kdiag rows are pivot rows (forward: D^-1 rows
 // that go to Y[ydiag + i]; backward: masked); xcol = first pivot column of the item in the subdomain's permuted numbering
@@ -64,7 +61,8 @@ class SolveForest {
   // plans[s] solves rows [xoff[s], xoff[s]+n_s) of the concatenated (permuted) vectors
   void build(const std::vector<const LdltPlan*>& plans, const std::vector<int64_t>& xoff);
   void set_factors(const std::vector<const double*>& L, cudaStream_t st);
-  // X (forward sweep, overwritten) -> Y (result); row-major blocks with leading dimension ldx, columns j0..j0+nr-1
+  // X (forward sweep, overwritten) -> Y (result); row-major blocks with leading dimension ldx, columns j0..j0+nr-1;
+  // nr = 8 or 16, or nr = 1 with ldx = 1
   void solve(double* X, double* Y, int ldx, int j0, int nr, cudaStream_t st) const;
   // NR = 1 solve with a device timestamp after every level barrier: us[p] = duration of phase p (forward levels bottom-up,
   // then backward levels top-down), bytes[p] = factor bytes streamed in it, nitems[p] = ring items
@@ -73,14 +71,10 @@ class SolveForest {
   int64_t ntot = 0;
  private:
   void build_ring(int which) const;  // which = 0: NR = 1 item lists, 1: NR = 8 (built on first use)
-  void build_generic() const;        // item lists of the generic kernels (nr = 2, 4; built on first use)
   std::vector<const LdltPlan*> plans_;
   std::vector<int64_t> xoff_;
   std::vector<ForestSub> hSubs;
   DevBuf<ForestSub> dSubs;
-  mutable DevBuf<ForestItem> dItems;
-  mutable DevBuf<int64_t> dRanges;
-  mutable bool genericBuilt = false;
   // ring kernels (NR = 1 and NR = 8): their own item lists (spans chosen per level) and ranges, built on first use
   mutable DevBuf<RingItem> dRing[2];
   mutable DevBuf<int64_t> dRingRanges[2];
@@ -88,8 +82,6 @@ class SolveForest {
   mutable std::vector<int64_t> ringCount_[2];
   mutable bool ringBuilt[2] = {false, false};
   int ringGrid[2] = {1, 1};
-  int ringVar = 0;  // tuning variant of the ring kernels (GENEO_RING_VAR when the forest was built)
-  int gridBlocks[4] = {1, 1, 1, 1};
 };
 
 struct FactorStats { int neg = 0, perturbed = 0; double seconds = 0.; };
@@ -109,7 +101,7 @@ class LdltFactor {
   // vals: device array aligned with the plan's input CSR pattern.  pivTol: a |pivot| below it is a null pivot, fixed to 1e34 pivTol (MUMPS CNTL(5) semantics).
   FactorStats factorize(const double* dVals, double pivTol, LdltWorkspace& ws, cudaStream_t st);
   // Solve in the PERMUTED ordering: X (n x ldx row-major block, columns j0..j0+nr-1) is overwritten by the forward
-  // sweep, the result lands in Y (same layout).  nr in {1,2,4,8,16}.
+  // sweep, the result lands in Y (same layout).  nr in {8, 16}, or nr = 1 with ldx = 1.
   void solve_permuted(double* X, double* Y, int ldx, int j0, int nr, cudaStream_t st) const;
   const LdltPlan& plan() const { return *plan_; }
   std::shared_ptr<LdltPlan> plan_ptr() const { return plan_; }

@@ -198,8 +198,9 @@ int geneo_host_sym_eig(int n, double* a /* row-major in, eigenvectors (columns) 
 int geneo_host_sym_eig_rows(int n, double* a, const int32_t* rows, int nrows, double* w, double* yrows);
 /* microbenchmarks on the device (first-run calibration): kind 0 = DMMA 64x64-tile GEMM C=AB^T (M=N=K=n) TFLOP/s,
  * kind 1 = device copy GB/s over n doubles, kind 2 = solve-kernel streaming over ~2 GB of synthetic n x 128 panels at a
- * single level (result[0] = algorithmic GB/s, result[1] = ms per solve).  result[0] = rate, result[1] = max abs error vs a
- * reference (kind 0). */
+ * single level (result[0] = algorithmic GB/s, result[1] = ms per solve), kind 100 * nlev + nr (nlev >= 1, nr = 1, 8 or 16;
+ * any other nr is rejected) = level-latency probe of the nr-column solve over nlev levels of `reps` n x 128 panels each
+ * (same results as kind 2).  result[0] = rate, result[1] = max abs error vs a reference (kind 0). */
 int geneo_microbench(int kind, int n, int reps, double result[2]);
 
 #ifdef __cplusplus

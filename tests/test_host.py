@@ -30,6 +30,13 @@ def test_no_cpu_fallback_without_device():
         g.microbench(1, 1024)
 
 
+def test_level_probe_rejects_a_block_width_without_a_solve_kernel():
+    """microbench kind 100 * nlev + nr: the solve kernels exist for nr = 1, 8 and 16 only.  The kind is checked before the
+    device is touched, so the same error comes with or without a GPU."""
+    with pytest.raises(g.GeneoError, match="nr must be 1, 8 or 16"):
+        g.microbench(102, 128, 1)
+
+
 @pytest.mark.parametrize("kind,args,kw", [
     ("laplacian", "--dim 3 --size 9 --kappa 2. lin --inpEps 0.0001", dict(dim=3, size=9, inp_eps=1e-4, kappa_max=2.0, interp="lin")),
     ("laplacian", "--dim 2 --size 11 --weakScaling 3 --kappa 5. quad", dict(dim=2, size=11, weak=3, kappa_max=5.0, interp="quad")),
