@@ -339,7 +339,7 @@ def box_ordering(dims, stencil=((1, 0, 0), (0, 1, 0), (0, 0, 1)), threads=1):
 class Symbolic:
     """Host-only view of the symbolic analysis (test hook)."""
 
-    def __init__(self, a_csr, nb=128, ordering=1, amalgamate=True, coords=None, perm=None):
+    def __init__(self, a_csr, nb=128, ordering=1, amalgamate=True, perm=None):
         a = a_csr.tocsr()
         self.n = a.shape[0]
         ptr = np.ascontiguousarray(a.indptr, dtype=np.int64)
@@ -349,10 +349,6 @@ class Symbolic:
             pp = np.ascontiguousarray(perm, dtype=np.int32)
             _chk(lib.geneo_symbolic_create_perm(C.c_int(self.n), _p(ptr, _i64p), _p(idx, _i32p), C.c_int(nb),
                                                 C.c_int(1 if amalgamate else 0), _p(pp, _i32p), C.byref(self.h)))
-        elif coords is not None:  # geometric nested dissection on integer vertex coordinates (n x 3)
-            xyz = np.ascontiguousarray(coords, dtype=np.int32).reshape(self.n, 3)
-            _chk(lib.geneo_symbolic_create_geo(C.c_int(self.n), _p(ptr, _i64p), _p(idx, _i32p), C.c_int(nb),
-                                               C.c_int(1 if amalgamate else 0), _p(xyz, _i32p), C.byref(self.h)))
         else:
             _chk(lib.geneo_symbolic_create(C.c_int(self.n), _p(ptr, _i64p), _p(idx, _i32p), C.c_int(nb), C.c_int(ordering),
                                            C.c_int(1 if amalgamate else 0), C.byref(self.h)))

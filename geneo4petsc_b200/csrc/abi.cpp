@@ -589,20 +589,10 @@ int geneo_symbolic_create(int n, const int64_t* ptr, const int32_t* idx, int nb,
                           geneo_symbolic_t* out) {
   ABI_TRY
   ABI_REQ(ptr && idx && out && n > 0, "null argument");
+  ABI_REQ(ordering == 0 || ordering == 1, "ordering must be 0 (natural) or 1 (METIS)");
   geneo_symbolic_s* s = new geneo_symbolic_s();
   SymbolicOptions o;
   o.nb = nb; o.ordering = ordering; o.amalgamate = amalgamate != 0;
-  try { symbolic_analyze(n, ptr, idx, o, s->s); } catch (...) { delete s; throw; }
-  *out = s;
-  ABI_CATCH
-}
-int geneo_symbolic_create_geo(int n, const int64_t* ptr, const int32_t* idx, int nb, int amalgamate, const int32_t* coords,
-                              geneo_symbolic_t* out) {
-  ABI_TRY
-  ABI_REQ(ptr && idx && out && coords && n > 0, "null argument");
-  geneo_symbolic_s* s = new geneo_symbolic_s();
-  SymbolicOptions o;
-  o.nb = nb; o.ordering = 2; o.amalgamate = amalgamate != 0; o.coords = coords;
   try { symbolic_analyze(n, ptr, idx, o, s->s); } catch (...) { delete s; throw; }
   *out = s;
   ABI_CATCH

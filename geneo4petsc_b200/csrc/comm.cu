@@ -17,7 +17,6 @@ enum { ncclSum = 0 };
 struct Api {
   int (*GetUniqueId)(NcclUid*) = nullptr;
   int (*CommInitRank)(ncclComm_t*, int, NcclUid, int) = nullptr;
-  int (*CommDestroy)(ncclComm_t) = nullptr;
   int (*AllReduce)(const void*, void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
   int (*Send)(const void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
   int (*Recv)(void*, size_t, int, int, ncclComm_t, cudaStream_t) = nullptr;
@@ -36,7 +35,6 @@ Api& api() {
   auto sym = [&](const char* n) { void* p = dlsym(h, n); if (!p) throw Error(std::string("geneo_b200: libnccl lacks ") + n); return p; };
   a.GetUniqueId = (decltype(a.GetUniqueId))sym("ncclGetUniqueId");
   a.CommInitRank = (decltype(a.CommInitRank))sym("ncclCommInitRank");
-  a.CommDestroy = (decltype(a.CommDestroy))sym("ncclCommDestroy");
   a.AllReduce = (decltype(a.AllReduce))sym("ncclAllReduce");
   a.Send = (decltype(a.Send))sym("ncclSend");
   a.Recv = (decltype(a.Recv))sym("ncclRecv");
@@ -77,22 +75,16 @@ inline int grid_for(int64_t n) { return (int)std::max<int64_t>(1, std::min<int64
 
 }  // namespace
 
-Comm::~Comm() { reset(); }
-
 // One NCCL communicator per PROCESS and (rank, world), shared by every preconditioner the process sets up -- the way MPI
 // hands the reference one PETSC_COMM_WORLD for all its PCs.  ncclCommInitRank and the lazily established peer connections of
 // the first send / recv / allreduce cost seconds on 8 GPUs; a second PCSetUp in the same job must not pay them again.
-// (GENEO_COMM_PER_PC=1: the old behaviour, a fresh communicator per setup.)
 namespace {
 struct SharedComm { int rank, world; ncclComm_t c; };
 std::vector<SharedComm>& shared_comms() { static std::vector<SharedComm>* v = new std::vector<SharedComm>(); return *v; }
-bool comm_per_pc() { static const bool v = getenv("GENEO_COMM_PER_PC") != nullptr; return v; }
 }  // namespace
 
 void Comm::reset() {
-  if (comm_ && owned_) api().CommDestroy((ncclComm_t)comm_);
   comm_ = nullptr;
-  owned_ = false;
   rank = 0; world = 1; nOwn = nGhost = 0; bufWidth_ = 0;
   sendPtr_.clear(); recvPtr_.clear();
 }
@@ -104,21 +96,19 @@ void Comm::unique_id(void* out128) {
 }
 
 void Comm::init(int rank_, int world_, const void* uid128, const RankLayout& L, cudaStream_t st) {
-  reset();  // a repeated setup gets a fresh communicator
+  reset();
   rank = rank_; world = world_;
   nOwn = L.nOwn(); nGhost = L.nGhost();
   if (world <= 1) return;
   GENEO_CHECK(uid128 != nullptr, "multi-GPU setup without an NCCL unique id");
   ncclComm_t c = nullptr;
-  if (!comm_per_pc())
-    for (auto& sc : shared_comms())
-      if (sc.rank == rank && sc.world == world) c = sc.c;  // (every rank takes the same branch: they all set up the same sequence of PCs)
+  for (auto& sc : shared_comms())
+    if (sc.rank == rank && sc.world == world) c = sc.c;  // (every rank takes the same branch: they all set up the same sequence of PCs)
   if (!c) {
     NcclUid id;
     std::memcpy(&id, uid128, sizeof(id));
     NCCL_CHECK(api().CommInitRank(&c, world, id, rank));
-    if (comm_per_pc()) owned_ = true;
-    else shared_comms().push_back(SharedComm{rank, world, c});
+    shared_comms().push_back(SharedComm{rank, world, c});
   }
   comm_ = c;
   sendPtr_.assign(world + 1, 0);

@@ -17,8 +17,7 @@ class Comm {
  public:
   int rank = 0, world = 1;
   bool active() const { return world > 1; }
-  ~Comm();
-  void reset();  // destroy the communicator, back to the single-process state
+  void reset();  // back to the single-process state (the process-wide communicator stays for the next init)
   static void unique_id(void* out128);  // ncclGetUniqueId (rank 0), to be broadcast by the caller
   void init(int rank, int world, const void* uid128, const RankLayout& L, cudaStream_t st);
   void allreduce_sum(double* d, int n, cudaStream_t st);      // in place, device buffer
@@ -30,8 +29,7 @@ class Comm {
   int nOwn = 0, nGhost = 0;
   int64_t bytesSent = 0;  // per-process NVLink traffic issued (statistics)
  private:
-  void* comm_ = nullptr;  // ncclComm_t
-  bool owned_ = false;    // false: the process-wide communicator of (rank, world), never destroyed by a PC
+  void* comm_ = nullptr;  // ncclComm_t: the process-wide communicator of (rank, world), never destroyed
   std::vector<int64_t> sendPtr_, recvPtr_;  // [world+1]: rows sent to / received from each peer
   DevBuf<int> dSendIdx_;
   DevBuf<double> sendBuf_, recvBuf_, tmp_;

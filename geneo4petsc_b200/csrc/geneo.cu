@@ -40,10 +40,7 @@ struct CachedBlock { void* p; size_t cap; };
 std::vector<CachedBlock>& g_dev_cache = *new std::vector<CachedBlock>();
 size_t g_dev_cache_bytes = 0;
 std::mutex& g_dev_cache_mtx = *new std::mutex();
-size_t dev_cache_limit() {
-  static const size_t lim = [] { const char* e = getenv("GENEO_CACHE_GB"); return (size_t)((e ? atof(e) : 16.) * 1073741824.); }();
-  return lim;
-}
+constexpr size_t DEV_CACHE_LIMIT = (size_t)16 << 30;  // bytes of freed blocks the cache keeps at most
 }  // namespace
 void dev_cache_flush() {
   std::lock_guard<std::mutex> lk(g_dev_cache_mtx);
@@ -83,7 +80,7 @@ void* dev_alloc(size_t bytes, size_t* cap) {
 void dev_free(void* p, size_t cap) {
   if (!p) return;
   std::lock_guard<std::mutex> lk(g_dev_cache_mtx);
-  if (cap > dev_cache_limit() / 2 || g_dev_cache_bytes + cap > dev_cache_limit() || g_dev_cache.size() >= 256) {
+  if (cap > DEV_CACHE_LIMIT / 2 || g_dev_cache_bytes + cap > DEV_CACHE_LIMIT || g_dev_cache.size() >= 256) {
     cudaFree(p);
     return;
   }
@@ -251,6 +248,7 @@ int GeneoOptions::parse(int argc, const char* const* argv, std::string& err) {
   if (lvl2 >= 1 && tau >= 1.) { err = "GenEO preconditioner: tau must be < 1."; return 1; }
   if (lvl2 >= 2 && gamma <= 1.) { err = "GenEO preconditioner: gamma must be > 1."; return 1; }
   if (nb < 8 || nb > 128) { err = "-geneo_nb must be in [8,128]"; return 1; }
+  if (ordering != 0 && ordering != 1) { err = "-geneo_ordering must be 0 (natural) or 1 (METIS)"; return 1; }
   return 0;
 }
 
@@ -1480,7 +1478,6 @@ void GeneoPC::numeric_pipeline() {
   }
   const bool history = l2 && prevMaxNev > 0;
   int want = std::min(P, (history || !l2) ? 4 : 2);
-  if (const char* e = getenv("GENEO_LANES")) want = std::max(1, std::min(P, atoi(e)));
   {
     size_t freeB = 0, totB = 0;
     CUDA_CHECK(cudaMemGetInfo(&freeB, &totB));
@@ -1626,7 +1623,6 @@ void GeneoPC::numeric_pipeline() {
   // ---- the eigen-solves, one lane group at a time: the pencils of a group run in LOCK-STEP (one host thread each, one
   //      forest solve per step over the group's shift-invert factors) while the helper keeps the lanes busy with the
   //      level-1 factorizations of this group and the S / A_neu factorizations of the next one
-  static const bool groupEig = getenv("GENEO_GROUP_EIG") ? atoi(getenv("GENEO_GROUP_EIG")) != 0 : true;
   if ((int)groupSolvers.size() < (P + NL - 1) / NL) groupSolvers.resize((P + NL - 1) / NL);
   bool mainAbort = false;
   for (int g0 = 0; l2 && g0 < P && !mainAbort; g0 += NL) {
@@ -1654,7 +1650,7 @@ void GeneoPC::numeric_pipeline() {
     // Do the Lanczos buffers of all members fit at once?  (basis + its B image: 2 n maxDim doubles per pencil -- 20 GB for a
     // heat subdomain that wants 200 pairs.)  If not, the pencils run one after the other on the library's stream, as in
     // the sequential path, and share one workspace.
-    bool threaded = groupEig && act.size() >= 2 && !g_hostprof;
+    bool threaded = act.size() >= 2 && !g_hostprof;
     if (threaded) {
       double need = 0.;
       for (int p : act) {

@@ -4,8 +4,6 @@
 #include <dlfcn.h>
 
 #include <algorithm>
-#include <climits>
-#include <cmath>
 #include <numeric>
 #include <string>
 #include <thread>
@@ -62,29 +60,13 @@ namespace {
 
 struct NdGraph { std::vector<midx_t> xadj, adj; int n() const { return (int)xadj.size() - 1; } };
 
-void metis_opts(midx_t* options) {
-  METIS_SetDefaultOptions(options);
-  if (const char* e = getenv("GENEO_METIS_OPTS")) {  // "idx=val,idx=val" experiment hook
-    std::string str(e);
-    size_t pos = 0;
-    while (pos < str.size()) {
-      size_t c = str.find(',', pos);
-      if (c == std::string::npos) c = str.size();
-      const std::string kv = str.substr(pos, c - pos);
-      const size_t eq = kv.find('=');
-      if (eq != std::string::npos) options[atoi(kv.substr(0, eq).c_str())] = atoi(kv.substr(eq + 1).c_str());
-      pos = c + 1;
-    }
-  }
-}
-
 // Nested dissection with the top `depth` levels done here so that the two halves can be ordered concurrently
 // (METIS_NodeND is serial; its own recursion does exactly this: separator last, halves recursively).  order: new -> old.
 void nd_recursive(NdGraph& g, int depth, std::vector<int>& order) {
   NdRngScope rngScope;
   const int n = g.n();
   midx_t options[40];
-  metis_opts(options);
+  METIS_SetDefaultOptions(options);
   midx_t nv = n;
   if (depth <= 0 || n < 20000) {
     std::vector<midx_t> p(n), ip(n);
@@ -130,105 +112,6 @@ void nd_recursive(NdGraph& g, int depth, std::vector<int>& order) {
   for (int s = 0; s < 2; s++)
     for (int v : ord[s]) order.push_back(ids[s][v]);
   for (int v : ids[2]) order.push_back(v);
-}
-
-// Geometric nested dissection: every region is cut at the median coordinate of its longest axis; the separator is the
-// set of vertices of the upper half that touch the lower half (for a 7-point grid: exactly one plane of nodes), ordered
-// last.  Works on any graph whose vertices carry integer coordinates; O(nnz log n), no METIS call.  At 100^3 it costs
-// 0.3 s where METIS_NodeND needs 5-15 s of one core -- the host wall of the cold setup at 8 subdomains per GPU and 8
-// ranks per node -- and, being the textbook ordering of a regular grid, it gives regular separators (planes) and a
-// slightly smaller factor.  order: new -> old.
-void geometric_nd(int n, const int64_t* ptr, const int* idx, const int* coords, int leaf, std::vector<int>& order) {
-  std::vector<int> verts(n), tmp(n);
-  std::iota(verts.begin(), verts.end(), 0);
-  std::vector<int> side(n, -1);     // scratch: region stamp / side of the current cut
-  order.assign(n, -1);
-  struct Region { int b, e, outPos; };  // verts[b, e) -> order[outPos, outPos + (e - b))
-  std::vector<Region> stack;
-  stack.push_back(Region{0, n, 0});
-  std::vector<int> cnt;
-  int metisBelow = 0;
-  if (const char* e = getenv("GENEO_GEO_METIS_T")) metisBelow = atoi(e);
-  while (!stack.empty()) {
-    const Region R = stack.back();
-    stack.pop_back();
-    const int m = R.e - R.b;
-    if (m <= leaf) {
-      for (int t = 0; t < m; t++) order[R.outPos + t] = verts[R.b + t];
-      continue;
-    }
-    if (m <= metisBelow) {  // hybrid: the region's own graph goes to METIS_NodeND
-      NdRngScope rngScope;
-      for (int t = 0; t < m; t++) side[verts[R.b + t]] = t;  // local numbering
-      std::vector<midx_t> xadj(m + 1, 0), adj;
-      for (int t = 0; t < m; t++) {
-        const int v = verts[R.b + t];
-        for (int64_t e = ptr[v]; e < ptr[v + 1]; e++) { const int u = idx[e]; if (u != v && side[u] >= 0) adj.push_back(side[u]); }
-        xadj[t + 1] = (midx_t)adj.size();
-      }
-      for (int t = 0; t < m; t++) side[verts[R.b + t]] = -1;
-      if (adj.empty()) { for (int t = 0; t < m; t++) order[R.outPos + t] = verts[R.b + t]; continue; }
-      midx_t options[40];
-      metis_opts(options);
-      midx_t nv = m;
-      std::vector<midx_t> p(m), ip(m);
-      const int rc = METIS_NodeND(&nv, xadj.data(), adj.data(), NULL, options, p.data(), ip.data());
-      GENEO_CHECK(rc == 1, "METIS_NodeND failed");
-      for (int t = 0; t < m; t++) order[R.outPos + t] = verts[R.b + (int)p[t]];
-      continue;
-    }
-    int lo[3] = {INT32_MAX, INT32_MAX, INT32_MAX}, hi[3] = {INT32_MIN, INT32_MIN, INT32_MIN};
-    for (int t = R.b; t < R.e; t++)
-      for (int a = 0; a < 3; a++) {
-        const int c = coords[3 * (size_t)verts[t] + a];
-        lo[a] = std::min(lo[a], c); hi[a] = std::max(hi[a], c);
-      }
-    int ax = 0;
-    for (int a = 1; a < 3; a++) if (hi[a] - lo[a] > hi[ax] - lo[ax]) ax = a;
-    if (hi[ax] == lo[ax]) {  // all vertices at one point: nothing to cut
-      for (int t = 0; t < m; t++) order[R.outPos + t] = verts[R.b + t];
-      continue;
-    }
-    // cut coordinate: the smallest c with #{coord < c} >= m/2 (histogram over the extent)
-    cnt.assign((size_t)(hi[ax] - lo[ax]) + 2, 0);
-    for (int t = R.b; t < R.e; t++) cnt[coords[3 * (size_t)verts[t] + ax] - lo[ax] + 1]++;
-    int cut = lo[ax] + 1;
-    {
-      int64_t acc = 0;
-      for (int c = lo[ax]; c <= hi[ax]; c++) {
-        acc += cnt[c - lo[ax] + 1];
-        if (2 * acc >= m) { cut = c + 1; break; }
-      }
-      if (cut > hi[ax]) cut = hi[ax];
-    }
-    // side: 0 lower (coord < cut), 1 upper; separator = upper vertices with a lower neighbour INSIDE the region
-    for (int t = R.b; t < R.e; t++) side[verts[t]] = coords[3 * (size_t)verts[t] + ax] < cut ? 0 : 1;
-    int nl = 0, nu = 0, nsep = 0;
-    for (int t = R.b; t < R.e; t++) {
-      const int v = verts[t];
-      if (side[v] == 0) { nl++; continue; }
-      bool sep = false;
-      for (int64_t e = ptr[v]; e < ptr[v + 1] && !sep; e++) {
-        const int u = idx[e];
-        if (u != v && side[u] == 0) sep = true;
-      }
-      if (sep) side[v] = 2;
-    }
-    // stable three-way split of verts[b, e): lower | upper | separator
-    for (int t = R.b; t < R.e; t++) { const int s = side[verts[t]]; if (s == 1) nu++; else if (s == 2) nsep++; }
-    int pl = R.b, pu = R.b + nl, ps = R.b + nl + nu;
-    for (int t = R.b; t < R.e; t++) {
-      const int v = verts[t];
-      const int s = side[v];
-      tmp[s == 0 ? pl++ : (s == 1 ? pu++ : ps++)] = v;
-    }
-    std::copy(tmp.begin() + R.b, tmp.begin() + R.e, verts.begin() + R.b);
-    for (int t = R.b; t < R.e; t++) side[verts[t]] = -1;  // vertices outside the region must never look like "lower"
-    for (int t = 0; t < nsep; t++) order[R.outPos + nl + nu + t] = verts[R.b + nl + nu + t];
-    // (nsep == 0: no edge crosses the cut -- the halves are independent regions all the same)
-    if (nl > 0) stack.push_back(Region{R.b, R.b + nl, R.outPos});
-    if (nu > 0) stack.push_back(Region{R.b + nl, R.b + nl + nu, R.outPos + nl});
-  }
 }
 
 // Elimination tree of P A P^T (Liu, path compression).  Row j of the permuted matrix = row perm[j] of the input.
@@ -325,69 +208,23 @@ void box_reference_ordering(const int dims[3], int nst, const int* stencil, int 
       if ((a | b | c) == 0 || have(a, b, c)) continue;
       off.push_back(a); off.push_back(b); off.push_back(c);
     }
-  auto boxGraph = [&](const int d[3], NdGraph& g) {
-    const int nv = d[0] * d[1] * d[2];
-    g.xadj.assign((size_t)nv + 1, 0);
-    g.adj.clear();
-    g.adj.reserve((size_t)nv * (off.size() / 3));
-    for (int z = 0; z < d[2]; z++)
-      for (int y = 0; y < d[1]; y++)
-        for (int x = 0; x < d[0]; x++) {
-          const int v = x + d[0] * (y + d[1] * z);
-          for (size_t t = 0; t < off.size(); t += 3) {
-            const int a = x + off[t], b = y + off[t + 1], c = z + off[t + 2];
-            if (a < 0 || a >= d[0] || b < 0 || b >= d[1] || c < 0 || c >= d[2]) continue;
-            g.adj.push_back(a + d[0] * (b + d[1] * c));
-          }
-          g.xadj[(size_t)v + 1] = (midx_t)g.adj.size();
+  NdGraph g;
+  g.xadj.assign((size_t)n + 1, 0);
+  g.adj.reserve((size_t)n * (off.size() / 3));
+  for (int z = 0; z < dims[2]; z++)
+    for (int y = 0; y < dims[1]; y++)
+      for (int x = 0; x < dims[0]; x++) {
+        const int v = x + dims[0] * (y + dims[1] * z);
+        for (size_t t = 0; t < off.size(); t += 3) {
+          const int a = x + off[t], b = y + off[t + 1], c = z + off[t + 2];
+          if (a < 0 || a >= dims[0] || b < 0 || b >= dims[1] || c < 0 || c >= dims[2]) continue;
+          g.adj.push_back(a + dims[0] * (b + dims[1] * c));
         }
-  };
+        g.xadj[(size_t)v + 1] = (midx_t)g.adj.size();
+      }
   std::vector<int> order;
-  int reach = 0;  // widest coupling along any axis: the top plane must be that thick to separate the halves
-  for (size_t t = 0; t < off.size(); t++) reach = std::max(reach, std::abs(off[t]));
-  int axis = 0;
-  for (int a = 1; a < 3; a++) if (dims[a] > dims[axis]) axis = a;
-  if (const char* e = getenv("GENEO_BOX_TOP_AXIS")) axis = std::max(0, std::min(2, atoi(e)));
-  // (experiment, off by default: GENEO_BOX_TOP_PLANE=1 writes the top separator down as the mid-plane of the longest axis
-  //  instead of asking METIS -- 35 % less ordering time, but the halves then come out 2-7 % more expensive in flops than
-  //  when METIS cuts the whole box itself, measured at 100^3..102^3)
-  bool topPlane = false;
-  if (const char* e = getenv("GENEO_BOX_TOP_PLANE")) topPlane = atoi(e) != 0 && ndDepth >= 1 && n >= 20000 && reach == 1 && dims[axis] >= 8;
-  if (off.empty()) { order.resize(n); std::iota(order.begin(), order.end(), 0); }
-  else if (topPlane) {
-    // The smallest balanced vertex separator of a box of nearest-neighbour couplings is the mid-plane across its longest
-    // axis -- METIS_ComputeVertexSeparator finds a plane of that size on a cube, after 40 % of the whole ordering time
-    // spent serially on the 10^6-vertex graph.  Here it is written down; METIS orders the two halves (concurrently).
-    const int mid = dims[axis] / 2;
-    int dA[3] = {dims[0], dims[1], dims[2]}, dB[3] = {dims[0], dims[1], dims[2]};
-    dA[axis] = mid;
-    dB[axis] = dims[axis] - mid - 1;
-    NdGraph gA, gB;
-    std::vector<int> oA, oB;
-    std::string err;
-    std::thread th([&]() { try { boxGraph(dA, gA); nd_recursive(gA, ndDepth - 1, oA); } catch (std::exception& e) { err = e.what(); } });
-    boxGraph(dB, gB);
-    nd_recursive(gB, ndDepth - 1, oB);
-    th.join();
-    GENEO_CHECK(err.empty(), err);
-    auto globalId = [&](const int d[3], int shift, int v) {
-      int c[3] = {v % d[0], (v / d[0]) % d[1], v / (d[0] * d[1])};
-      c[axis] += shift;
-      return c[0] + dims[0] * (c[1] + dims[1] * c[2]);
-    };
-    order.reserve(n);
-    for (int v : oA) order.push_back(globalId(dA, 0, v));
-    for (int v : oB) order.push_back(globalId(dB, mid + 1, v));
-    for (int v = 0; v < n; v++) {
-      const int c[3] = {v % dims[0], (v / dims[0]) % dims[1], v / (dims[0] * dims[1])};
-      if (c[axis] == mid) order.push_back(v);
-    }
-  } else {
-    NdGraph g;
-    boxGraph(dims, g);
-    if (g.adj.empty()) { order.resize(n); std::iota(order.begin(), order.end(), 0); }
-    else nd_recursive(g, ndDepth, order);
-  }
+  if (g.adj.empty()) { order.resize(n); std::iota(order.begin(), order.end(), 0); }
+  else nd_recursive(g, ndDepth, order);
   GENEO_CHECK((int)order.size() == n, "reference box: nested dissection lost vertices");
   rank.assign(n, 0);
   for (int i = 0; i < n; i++) rank[order[i]] = i;
@@ -404,13 +241,7 @@ void symbolic_analyze(int n, const int64_t* ptr, const int* idx, const SymbolicO
 
   // ---- 1. fill-reducing ordering ------------------------------------------------------------------------------------
   std::vector<int> perm(n), iperm(n);
-  bool useMetis = ((opt.ordering == 1 || (opt.ordering == 2 && !opt.coords)) && n > 32);
-  bool useGeo = opt.ordering == 2 && opt.coords && n > 32;
-  if (useGeo) {
-    std::vector<int> order;
-    geometric_nd(n, ptr, idx, opt.coords, std::max(1, opt.geoLeaf), order);
-    for (int i = 0; i < n; i++) { GENEO_CHECK(order[i] >= 0, "geometric nested dissection lost vertices"); perm[i] = order[i]; iperm[order[i]] = i; }
-  }
+  bool useMetis = opt.ordering == 1 && n > 32;
   if (useMetis) {
     std::vector<midx_t> xadj(n + 1, 0), adj;
     adj.reserve(ptr[n]);
@@ -425,9 +256,7 @@ void symbolic_analyze(int n, const int64_t* ptr, const int* idx, const SymbolicO
       g.xadj.swap(xadj);
       g.adj.swap(adj);
       std::vector<int> order;
-      int depth = opt.ndDepth;
-      if (const char* e = getenv("GENEO_ND_DEPTH")) depth = atoi(e);
-      nd_recursive(g, depth, order);
+      nd_recursive(g, opt.ndDepth, order);
       GENEO_CHECK((int)order.size() == n, "nested dissection lost vertices");
       for (int i = 0; i < n; i++) { perm[i] = order[i]; iperm[order[i]] = i; }
     }
@@ -440,8 +269,7 @@ void symbolic_analyze(int n, const int64_t* ptr, const int* idx, const SymbolicO
       GENEO_CHECK(o >= 0 && o < n && iperm[o] < 0, "user permutation is not a permutation");
       perm[i] = o; iperm[o] = i;
     }
-  } else
-  if (!useMetis && !useGeo) { std::iota(perm.begin(), perm.end(), 0); std::iota(iperm.begin(), iperm.end(), 0); }
+  } else if (!useMetis) { std::iota(perm.begin(), perm.end(), 0); std::iota(iperm.begin(), iperm.end(), 0); }
 
   const bool tm = getenv("GENEO_SYM_TIMING") != nullptr;
   double tq = now_s();
@@ -495,8 +323,6 @@ void symbolic_analyze(int n, const int64_t* ptr, const int* idx, const SymbolicO
       subCols[s] += snK[s];
       if (snParent[s] != -1) subCols[snParent[s]] += subCols[s];
     }
-    int subtreeLimit = opt.subtreeCols;
-    if (const char* e = getenv("GENEO_SUBTREE_COLS")) subtreeLimit = atoi(e);
     for (int s = 0; s < ns; s++) {
       while (true) {
         int c = prev[s];
@@ -508,7 +334,7 @@ void symbolic_analyze(int n, const int64_t* ptr, const int* idx, const SymbolicO
         const double total = newk * newh - newk * (newk - 1.) / 2.;
         const double frac = z / total;
         bool merge = (newk <= 4) || (newk <= 16 && frac < 0.8) || (newk <= 48 && frac < 0.1) || (frac < 0.05) ||
-                     (subCols[s] <= subtreeLimit);
+                     (subCols[s] <= opt.subtreeCols);
         if (!merge) break;
         snFirst[s] = snFirst[c]; snK[s] = (int)newk; snH[s] = (int)newh; zeros[s] = z;
         alive[c] = 0; mergedInto[c] = s; prev[s] = prev[c];
@@ -650,14 +476,14 @@ void symbolic_analyze(int n, const int64_t* ptr, const int* idx, const SymbolicO
       if (m > 0) {
         F.wOff = w; w += m * F.k;
         w = (w + 15) & ~(int64_t)15;  // 128-byte alignment of every scratch panel / fresh update matrix
-        const bool inplace = opt.chainInplace && f > 0 && S.fronts[f - 1].chain && S.fronts[f - 1].parent == f;
+        const bool inplace = f > 0 && S.fronts[f - 1].chain && S.fronts[f - 1].parent == f;
         if (inplace) {
           const Front& C = S.fronts[f - 1];
           F.inplace = 1;
           F.uArena = C.uArena;
           F.uLd = C.uLd;
           F.uOff = C.uOff + (int64_t)F.k * ((int64_t)C.uLd + 1);
-        } else if (opt.chainInplace && F.chain) {  // first panel of a chain: lives until the tree parent of the last panel
+        } else if (F.chain) {  // first panel of a chain: lives until the tree parent of the last panel
           int last = f;
           while (S.fronts[last].chain) last++;
           const int lEnd = S.fronts[last].level + 1;
@@ -682,17 +508,16 @@ void symbolic_analyze(int n, const int64_t* ptr, const int* idx, const SymbolicO
     S.wArena = std::max(S.wArena, w);
   }
 
-  if (opt.chainInplace && opt.chainPairs)
-    for (int f = 0; f < nf; f++) {  // chains start at a fresh front followed by in-place panels: pair them up two by two
-      if (!(S.fronts[f].chain && !S.fronts[f].inplace && S.fronts[f].m() > 0)) continue;
-      int last = f;
-      while (S.fronts[last].chain) last++;
-      for (int i = f; i + 1 <= last; i += 2) {
-        if (!S.fronts[i + 1].inplace) break;
-        S.fronts[i].pair = 1;
-        S.fronts[i + 1].pair = 2;
-      }
+  for (int f = 0; f < nf; f++) {  // chains start at a fresh front followed by in-place panels: pair them up two by two
+    if (!(S.fronts[f].chain && !S.fronts[f].inplace && S.fronts[f].m() > 0)) continue;
+    int last = f;
+    while (S.fronts[last].chain) last++;
+    for (int i = f; i + 1 <= last; i += 2) {
+      if (!S.fronts[i + 1].inplace) break;
+      S.fronts[i].pair = 1;
+      S.fronts[i + 1].pair = 2;
     }
+  }
 
   lap("fronts+levels");
   // ---- 7. scatter map of the input values (lower triangle of P A P^T) into the panels --------------------------------

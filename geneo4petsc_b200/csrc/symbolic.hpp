@@ -2,8 +2,8 @@
 // (reference call sites: src/geneo.cpp:94-124 directLocalSolve, :452-500 getInertia, :746-780 buildEigenSolver).
 //
 // Design (B200-first, see DESIGN.md "Sparse LDL^T"):
-//   * fill-reducing ordering: METIS NodeND on the host, or an O(n log n) geometric nested dissection (coordinate
-//     bisection + vertex separator taken from the cut) when the caller knows vertex coordinates (structured generators);
+//   * fill-reducing ordering: METIS NodeND on the host, the natural order, or a permutation from the caller (the reference
+//     box ordering shared by the subdomains of a structured problem);
 //   * elimination tree, postorder, Gilbert-Ng-Peyton column counts, supernodes with relaxed amalgamation;
 //   * every supernode is cut into PANELS ("fronts") of at most NB pivot columns, chained in the assembly tree, so that
 //     each front needs exactly one dense NBxNB pivot-block inversion, one panel product and one Schur GEMM;
@@ -71,14 +71,9 @@ struct Symbolic {
 
 struct SymbolicOptions {
   int nb = 128;        // panel width
-  int ordering = 1;    // 0 natural, 1 METIS NodeND, 2 geometric nested dissection (needs coords; falls back to 1 without),
-                       // 3 caller-supplied permutation (userPerm)
+  int ordering = 1;    // 0 natural, 1 METIS NodeND, 3 caller-supplied permutation (userPerm)
   const int* userPerm = nullptr;  // ordering == 3: new -> old, length n
-  const int* coords = nullptr;  // optional: 3 integer coordinates per vertex (structured generators, SymbolicOptions::ordering == 2)
-  int geoLeaf = 48;    // geometric ND stops at regions of at most this many vertices
   bool amalgamate = true;
-  bool chainInplace = true;  // update matrices of supernode chains stay in place (see Front::inplace)
-  bool chainPairs = true;    // rank-256 trailing updates along in-place chains (see Front::pair)
   int subtreeCols = 64; // subtrees of the assembly tree with at most this many columns are merged into one dense front
   bool skipAsm = false;  // leave asmSrc / asmDst empty: the caller builds the scatter map itself (symbolic_asm_map, or
                          // fused with its own pass over the matrix as GeneoPC's host preparation does)

@@ -168,11 +168,9 @@ int geneo_allreduce_sum(geneo_pc_t pc, double* h, int n); /* host array, in plac
  * Host-only test hooks (no device needed): symbolic analysis of a CSR pattern, dense symmetric eigen-solver
  * ------------------------------------------------------------------------------------------------------------------ */
 typedef struct geneo_symbolic_s* geneo_symbolic_t;
+/* ordering: 0 natural, 1 METIS nested dissection */
 int geneo_symbolic_create(int n, const int64_t* ptr, const int32_t* idx, int nb, int ordering, int amalgamate,
                           geneo_symbolic_t* out);
-/* same with ordering = geometric nested dissection on integer vertex coordinates (coords[3*n]; structured generators) */
-int geneo_symbolic_create_geo(int n, const int64_t* ptr, const int32_t* idx, int nb, int amalgamate, const int32_t* coords,
-                              geneo_symbolic_t* out);
 /* same with a caller-supplied permutation (new -> old) */
 int geneo_symbolic_create_perm(int n, const int64_t* ptr, const int32_t* idx, int nb, int amalgamate, const int32_t* perm,
                                geneo_symbolic_t* out);

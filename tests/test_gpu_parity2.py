@@ -150,7 +150,6 @@ def test_sequential_and_pipelined_numeric_setup_agree(monkeypatch):
     monkeypatch.setenv("GENEO_PIPELINE", "0")
     seq = g.GeneoPC(argv).setup(p)
     monkeypatch.setenv("GENEO_PIPELINE", "1")
-    monkeypatch.setenv("GENEO_LANES", "3")
     pip = g.GeneoPC(argv).setup(p)
     assert [seq.sub_info(s)["nev"] for s in range(nparts)] == [pip.sub_info(s)["nev"] for s in range(nparts)]
     assert [seq.sub_info(s)["neg"] for s in range(nparts)] == [pip.sub_info(s)["neg"] for s in range(nparts)] == [0] * nparts

@@ -53,9 +53,12 @@ def test_structured_generator_matches_reference_element_sequence(kind, args, kw)
 
 def test_bad_options_are_rejected():
     for bad in (["-geneo_lvl", "FOO,1"], ["-geneo_lvl", "ASM,9"], ["-geneo_tau", "1.5"], ["-geneo_tau", "abc"],
-                ["-geneo_lvl", "SORAS,2", "-geneo_gamma", "0.5"], ["-geneo_lvl"]):
+                ["-geneo_lvl", "SORAS,2", "-geneo_gamma", "0.5"], ["-geneo_lvl"], ["-geneo_ordering", "2"],
+                ["-geneo_ordering", "-1"]):
         with pytest.raises(g.GeneoError):
             g.GeneoPC(bad)
+    with pytest.raises(g.GeneoError, match="ordering must be 0"):
+        g.Symbolic(sp.identity(40, format="csr"), ordering=2)
     assert g.GeneoPC(["-geneo_lvl", "SORAS,H2"]).name == "geneo2HSORAS"
     assert g.GeneoPC().name == "geneo1ASM"
     assert g.GeneoPC(["-geneo_lvl", "RAS,E1"]).name == "geneo1ERAS"
@@ -397,21 +400,6 @@ def test_host_preparation_fast_and_general_paths_agree():
     assert d3 == d4
 
 
-def test_geometric_nested_dissection_is_a_valid_ordering():
-    """-geneo_ordering 2 (coordinate bisection, separators from the cut): O(n log n), no METIS call; a valid permutation whose
-    symbolic structures drive a correct factorization."""
-    d = (9, 8, 7)
-    a = _box_matrix(d)
-    x = np.arange(d[0] * d[1] * d[2])
-    xyz = np.stack([x % d[0], (x // d[0]) % d[1], x // (d[0] * d[1])], axis=1)
-    sym = g.Symbolic(a, nb=8, coords=xyz)
-    assert sorted(sym.perm.tolist()) == list(range(a.shape[0]))
-    L, neg = _emul.factorize(sym, a.data)
-    assert neg == 0
-    b = np.random.default_rng(2).standard_normal(a.shape[0])
-    assert np.linalg.norm(a @ _emul.solve(sym, L, b) - b) <= 1e-9 * np.linalg.norm(b)
-
-
 def test_reference_plot_script_parses_the_cli_log():
     """tst/plot.py (the reference's post-processing, :56-116) must read the logs of the PETSc-free driver: its own `job` parser
     is imported from /root/reference (matplotlib stubbed out) and fed a log of geneo4petsc_b200/geneo4PETSc captured on the B200
@@ -488,21 +476,3 @@ def test_decomposition_of_a_mesh_that_does_not_hold_every_node_id():
         for t in range(3):
             assert np.array_equal(p.sub_intersect(s, t), q.sub_intersect(s, t))
 
-
-def test_mid_plane_top_separator_experiment_gives_a_valid_ordering(monkeypatch):
-    """GENEO_BOX_TOP_PLANE=1 (off by default): the reference box is cut by the mid-plane of its longest axis and METIS orders
-    the halves.  Still a permutation, the plane comes last, and the fill stays within 15 % of the all-METIS ordering."""
-    from geneo4petsc_b200.api import box_ordering
-    dims = (30, 28, 27)
-    base = box_ordering(dims, threads=4)
-    monkeypatch.setenv("GENEO_BOX_TOP_PLANE", "1")
-    rank = box_ordering(dims, threads=4)
-    n = dims[0] * dims[1] * dims[2]
-    assert sorted(rank.tolist()) == list(range(n)) and not np.array_equal(rank, base)
-    x = np.arange(n) % dims[0]
-    plane = np.flatnonzero(x == dims[0] // 2)
-    assert sorted(rank[plane].tolist()) == list(range(n - len(plane), n))  # the separator is eliminated last
-    a = _box_matrix(dims)
-    f0 = g.Symbolic(a, nb=32, perm=np.argsort(base).astype(np.int32)).info["flops"]
-    f1 = g.Symbolic(a, nb=32, perm=np.argsort(rank).astype(np.int32)).info["flops"]
-    assert f1 <= 1.15 * f0
