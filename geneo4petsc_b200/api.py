@@ -200,6 +200,13 @@ class GeneoPC:
         _chk(lib.geneo_pc_refactor(self.h))
         return self
 
+    def update(self, problem):
+        """PCSetUp with SAME_NONZERO_PATTERN: the values of `problem` (same partition, node sets and patterns as the last
+        setup) replace the resident ones, then the numeric setup runs.  A mismatch raises and leaves the PC as it was."""
+        self.problem = problem  # borrowed by the library: keep it alive
+        _chk(lib.geneo_pc_update(self.h, problem.h))
+        return self
+
     def level_profile(self):
         """(us, bytes, items) per phase of one level-1 solve: forward levels leaves-first, then backward root-first."""
         n = C.c_int()

@@ -22,6 +22,7 @@ struct geneo_problem_s {
 struct geneo_pc_s {
   GeneoPC pc;
   bool ready = false;
+  bool dist = false;  // set up by geneo_pc_setup_dist
   const geneo_problem_s* prob = nullptr;  // borrowed (like pcA / pcMap in the reference, src/geneo.cpp:2221-2230)
 };
 struct geneo_symbolic_s { Symbolic s; };
@@ -276,6 +277,7 @@ int geneo_pc_setup(geneo_pc_t pc, geneo_problem_t p) {
   ABI_REQ(p && p->decomposed, "GenEO preconditioner without a decomposed problem");
   require_device();
   pc->prob = p;
+  pc->dist = false;
   pc->pc.setup(p->dec);
   pc->ready = true;
   ABI_CATCH
@@ -354,6 +356,7 @@ int geneo_pc_setup_dist(geneo_pc_t pc, geneo_problem_t p, geneo_layout_t l, cons
   ABI_REQ(pc && p && p->decomposed && l, "GenEO preconditioner without a decomposed problem / layout");
   require_device();
   pc->prob = p;
+  pc->dist = true;
   pc->pc.setup(p->dec, &l->L, ncclUid128);
   pc->ready = true;
   ABI_CATCH
@@ -377,6 +380,21 @@ int geneo_pc_refactor(geneo_pc_t pc) {
   ABI_TRY
   ABI_REQ(pc && pc->ready, "GenEO preconditioner without context");
   pc->pc.numeric_setup();
+  ABI_CATCH
+}
+int geneo_pc_update(geneo_pc_t pc, geneo_problem_t p) {
+  ABI_TRY
+  ABI_REQ(pc && pc->ready, "GenEO preconditioner without context");
+  ABI_REQ(p && p->decomposed, "GenEO preconditioner without a decomposed problem");
+  ABI_REQ(!pc->dist, "same-pattern update of a multi-GPU preconditioner (geneo_pc_setup_dist) is not supported: set it up again");
+  require_device();
+  GeneoPC::PendingValues nv;
+  pc->pc.check_values(p->dec, nv);  // throws on any mismatch before a resident value changes: the PC stays as it was
+  pc->ready = false;                // from here on values and factors disagree until the numeric setup has completed
+  pc->prob = p;
+  pc->pc.commit_values(nv);
+  pc->pc.numeric_setup();
+  pc->ready = true;
   ABI_CATCH
 }
 int geneo_pc_kernel_time(geneo_pc_t pc, double* ms, int64_t* launches) {

@@ -907,6 +907,7 @@ void GeneoPC::setup(const Decomposition& dec, const RankLayout* layout, const vo
     }
     s.maxMult = H.maxMult;
     s.anorm = H.anorm;
+    s.neuNnz = mine[p]->aNeu.nnz();
     s.plan = H.plan;
     s.plan->upload();
     s.pat.upload_pattern(H.patP, st);
@@ -1111,6 +1112,106 @@ void GeneoPC::numeric_setup() {
   numericTime = now_s() - tNum0;
   host_prof_add("numeric_setup total", numericTime);
   host_prof_report("numeric_setup");
+}
+
+// Same-pattern update.  Everything the setup derived from the pattern stays: plans (dPerm), the permuted A_dir pattern,
+// gidx, d, the operator's SELL layout, lanes and workspaces.  Per subdomain the new CSR matrices go up through one staging
+// set sized for the largest subdomain and are located on the device in the setup's pattern; the values land in fresh
+// buffers (PendingValues), and the counters of every check are read back once.  Only commit_values() writes resident values.
+void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv) {
+  require_device();
+  const int P = (int)subs.size();
+  GENEO_CHECK(P > 0 && !comm.active(), "update: the preconditioner is not set up on one process");
+  auto fail = [](const std::string& m) { throw Error("geneo_b200: same-pattern update: " + m); };
+  if (dec.nbPart != nbPart)
+    fail("the problem has " + std::to_string(dec.nbPart) + " subdomains, the preconditioner was set up with " + std::to_string(nbPart));
+  if (dec.nbNode != nbDof)
+    fail("the problem has " + std::to_string(dec.nbNode) + " DOFs, the preconditioner was set up with " + std::to_string(nbDof));
+  int nMax = 0;
+  int64_t zMax = 0;
+  for (int p = 0; p < P; p++) {
+    const Subdomain& S = dec.subs[p];
+    const SubdomainState& s = subs[p];
+    const std::string sub = "subdomain " + std::to_string(s.id) + ": ";
+    if (S.id != s.id || (int)S.nodes.size() != s.n) fail(sub + "the node set differs from the setup's (another partition?)");
+    if (S.aNeu.n != s.n || S.aDir.n != s.n) fail(sub + "no matrices on this process");
+    if (S.aDir.nnz() != s.pat.nnz)
+      fail(sub + "A_dir has " + std::to_string(S.aDir.nnz()) + " entries, the pattern of the setup " + std::to_string(s.pat.nnz));
+    if (S.aNeu.nnz() != s.neuNnz)
+      fail(sub + "A_neu has " + std::to_string(S.aNeu.nnz()) + " entries, the pattern of the setup " + std::to_string(s.neuNnz));
+    nMax = std::max(nMax, s.n);
+    zMax = std::max(zMax, s.pat.nnz);
+  }
+  CUDA_CHECK(::geneo::sync_stream(st));
+  DevBuf<int64_t> dPtr((size_t)nMax + 1);
+  DevBuf<int> dIdx((size_t)zMax), dNodes((size_t)nMax), dIperm((size_t)nMax), hits((size_t)zMax);
+  DevBuf<double> dVal((size_t)zMax);
+  DevBuf<unsigned long long> cnt((size_t)P * UPD_SLOTS + 1);  // + the operator entries no A_neu reached
+  DevBuf<unsigned char> cover((size_t)A.stored);
+  cnt.zero(st);
+  cover.zero(st);
+  nv.subs.clear();
+  nv.subs.resize(P);
+  for (int p = 0; p < P; p++) {
+    const Subdomain& S = dec.subs[p];
+    SubdomainState& s = subs[p];
+    const int n = s.n;
+    const int64_t nnz = s.pat.nnz, nnzNeu = s.neuNnz;
+    unsigned long long* c = cnt.p + (size_t)p * UPD_SLOTS;
+    PendingValues::Sub& w = nv.subs[p];
+    w.dir.alloc((size_t)nnz);
+    w.neu.alloc((size_t)nnz);
+    w.slot.alloc((size_t)nnz);
+    w.neu.zero(st);
+    CUDA_CHECK(cudaMemsetAsync(w.slot.p, 0xff, (size_t)nnz * sizeof(int64_t), st));  // -1: off the A_neu pattern
+    CUDA_CHECK(cudaMemsetAsync(hits.p, 0, (size_t)nnz * sizeof(int), st));
+    dNodes.upload(S.nodes.data(), (size_t)n, st);
+    update_nodes(n, s.plan->dPerm.p, s.gidx.p, dNodes.p, dIperm.p, c, st);
+    dPtr.upload(S.aDir.ptr.data(), (size_t)n + 1, st);
+    dIdx.upload(S.aDir.idx.data(), (size_t)nnz, st);
+    dVal.upload(S.aDir.val.data(), (size_t)nnz, st);
+    update_locate_dir(n, nnz, dPtr.p, dIdx.p, dVal.p, dIperm.p, s.pat.ptr.p, s.pat.idx.p, hits.p, w.dir.p, c, st);
+    update_absmax(nnz, w.dir.p, c + UPD_ANORM, st);
+    dPtr.upload(S.aNeu.ptr.data(), (size_t)n + 1, st);
+    dIdx.upload(S.aNeu.idx.data(), (size_t)nnzNeu, st);
+    dVal.upload(S.aNeu.val.data(), (size_t)nnzNeu, st);
+    update_locate_neu(n, nnzNeu, dPtr.p, dIdx.p, dVal.p, dIperm.p, s.gidx.p, s.pat.ptr.p, s.pat.idx.p, hits.p, A, w.neu.p, w.slot.p,
+                      cover.p, c, st);
+  }
+  update_cover_check(A, cover.p, cnt.p + (size_t)P * UPD_SLOTS, st);
+  const std::vector<unsigned long long> h = cnt.to_host(st);  // the only read-back
+  static const char* what[UPD_ANORM] = {
+      "node ids differ from the setup's", "A_dir rows whose length differs from the setup's", "A_dir entries outside the setup's pattern",
+      "duplicate A_dir entries", "A_neu entries outside the A_dir pattern", "duplicate A_neu entries",
+      "A_neu entries outside the operator's pattern"};
+  for (int p = 0; p < P; p++)
+    for (int e = 0; e < UPD_ANORM; e++)
+      if (h[(size_t)p * UPD_SLOTS + e])
+        fail("subdomain " + std::to_string(subs[p].id) + ": " + std::to_string(h[(size_t)p * UPD_SLOTS + e]) + " " + what[e]);
+  if (h[(size_t)P * UPD_SLOTS]) fail(std::to_string(h[(size_t)P * UPD_SLOTS]) + " entries of the operator are in no subdomain's A_neu");
+  for (int p = 0; p < P; p++) memcpy(&nv.subs[p].anorm, &h[(size_t)p * UPD_SLOTS + UPD_ANORM], sizeof(double));
+}
+
+// The checked values replace the resident ones.  Operator: zero, then + A_neu,p subdomain by subdomain in ascending order --
+// the host merge of setup() sums 0 + a_1 + a_2 ... in the same order, so A, mult() and everything downstream match a fresh
+// setup bit for bit.
+void GeneoPC::commit_values(PendingValues& nv) {
+  GENEO_CHECK(nv.subs.size() == subs.size(), "commit_values: the pending values do not belong to this preconditioner");
+  CUDA_CHECK(cudaMemsetAsync(A.val.p, 0, A.val.bytes(), st));
+  for (size_t p = 0; p < subs.size(); p++) {
+    SubdomainState& s = subs[p];
+    PendingValues::Sub& w = nv.subs[p];
+    s.anorm = w.anorm;
+    s.pat.val = std::move(w.dir);
+    s.vNeu = std::move(w.neu);
+    update_sell_add(s.pat.nnz, w.slot.p, s.vNeu.p, A, st);
+    if (opt.lvl1ORAS) {  // createRobinMatrix, as prepare_subdomain does it
+      if ((int64_t)s.vRob.n != s.pat.nnz) s.vRob.alloc((size_t)s.pat.nnz);
+      if (std::fabs(opt.optim) > DBL_EPSILON) update_robin(s.n, s.pat.ptr.p, s.pat.idx.p, s.d.p, s.pat.val.p, s.vNeu.p, opt.optim, s.vRob.p, st);
+      else CUDA_CHECK(cudaMemcpyAsync(s.vRob.p, s.pat.val.p, s.pat.val.bytes(), cudaMemcpyDeviceToDevice, st));
+    }
+  }
+  CUDA_CHECK(::geneo::sync_stream(st));
 }
 
 void GeneoPC::level_profile(std::vector<double>& us, std::vector<double>& bytes, std::vector<int64_t>& nitems) {

@@ -62,6 +62,7 @@ struct SubdomainState {
   double tauLoc = -1., gammaLoc = -1.;
   int maxMult = 1;
   double anorm = 0.;  // max |a_ij| of A_dir (scale of the static pivot threshold)
+  int64_t neuNnz = 0; // entries of the A_neu input (check_values: a same-pattern update has as many)
 };
 
 struct KspResult {
@@ -113,6 +114,17 @@ class GeneoPC {
   // Numeric half of the setup again (every factorization, eigen-solve, Z, E) on the matrices already resident in HBM:
   // PCSetUp with an unchanged non-zero pattern.  setup() = host analysis + uploads + numeric_setup().
   void numeric_setup();
+  // PCSetUp with SAME_NONZERO_PATTERN and new values (single process), in three steps: check_values() uploads the A_dir /
+  // A_neu values of `dec` -- same partition, node sets and patterns as the last setup() -- locates them in the resident
+  // pattern and checks them on the device without writing any resident value (on a mismatch it throws and the
+  // preconditioner is left as it was); commit_values() puts them in place (A_dir, A_neu, the Robin values, the operator,
+  // the pivot scale); numeric_setup() must follow before the next apply.
+  struct PendingValues {
+    struct Sub { DevBuf<double> dir, neu; DevBuf<int64_t> slot; double anorm = 0.; };  // slot: operator entry of A_neu q, or -1
+    std::vector<Sub> subs;
+  };
+  void check_values(const Decomposition& dec, PendingValues& nv);
+  void commit_values(PendingValues& nv);
   void numeric_begin();
   void numeric_end();
   // accumulated CUDA-event time of the level-1 solve kernel since the last call (ms) and its number of launches

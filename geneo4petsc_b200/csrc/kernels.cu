@@ -395,6 +395,111 @@ __global__ void __launch_bounds__(256) k_sum_all(int64_t nnz, const double* __re
   block_reduce_atomic<1>(s, out);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// same-pattern value update
+// ---------------------------------------------------------------------------------------------------------------
+// position of `key` among a[base + j * stride], j < len (ascending), or -1
+__device__ __forceinline__ int64_t find_sorted(const int* __restrict__ a, int64_t base, int64_t len, int stride, int key) {
+  int64_t lo = 0, hi = len;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (a[base + mid * stride] < key) lo = mid + 1;
+    else hi = mid;
+  }
+  return (lo < len && a[base + lo * stride] == key) ? base + lo * stride : -1;
+}
+__global__ void k_update_nodes(int n, const int* __restrict__ perm, const int* __restrict__ gidx, const int* __restrict__ nodes,
+                               int* __restrict__ iperm, unsigned long long* cnt) {
+  for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) {
+    const int r = perm[k];
+    iperm[r] = (int)k;
+    if (gidx[k] != nodes[r]) atomicAdd(cnt + UPD_NODES, 1ull);
+  }
+}
+__global__ void k_update_locate_dir(int n, int64_t nnz, const int64_t* __restrict__ ptr, const int* __restrict__ idx,
+                                    const double* __restrict__ val, const int* __restrict__ iperm, const int64_t* __restrict__ patPtr,
+                                    const int* __restrict__ patIdx, int* __restrict__ hits, double* __restrict__ dir,
+                                    unsigned long long* cnt) {
+  for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < n; r += (int64_t)gridDim.x * blockDim.x) {
+    const int k = iperm[r];
+    const int64_t a = ptr[r], b = ptr[r + 1], p0 = patPtr[k], len = patPtr[k + 1] - p0;
+    if (a < 0 || b > nnz || b - a != len) { atomicAdd(cnt + UPD_DIR_ROW, 1ull); continue; }
+    for (int64_t t = a; t < b; t++) {
+      const int c = idx[t];
+      const int64_t q = (c >= 0 && c < n) ? find_sorted(patIdx, p0, len, 1, iperm[c]) : -1;
+      if (q < 0) atomicAdd(cnt + UPD_DIR_OUTSIDE, 1ull);
+      else if (atomicOr(hits + q, 1) & 1) atomicAdd(cnt + UPD_DIR_DUP, 1ull);
+      else dir[q] = val[t];
+    }
+  }
+}
+__global__ void k_update_locate_neu(int n, int64_t nnz, const int64_t* __restrict__ ptr, const int* __restrict__ idx,
+                                    const double* __restrict__ val, const int* __restrict__ iperm, const int* __restrict__ gidx,
+                                    const int64_t* __restrict__ patPtr, const int* __restrict__ patIdx, int* __restrict__ hits,
+                                    const int64_t* __restrict__ sliceOff, const int* __restrict__ col, const int* __restrict__ rowLen,
+                                    double* __restrict__ neu, int64_t* __restrict__ slot, unsigned char* __restrict__ cover,
+                                    unsigned long long* cnt) {
+  for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < n; r += (int64_t)gridDim.x * blockDim.x) {
+    const int k = iperm[r];
+    const int64_t a = ptr[r], b = ptr[r + 1], p0 = patPtr[k], len = patPtr[k + 1] - p0;
+    if (a < 0 || b < a || b > nnz) { atomicAdd(cnt + UPD_NEU_OUTSIDE, 1ull); continue; }
+    const int g = gidx[k];  // row of the operator: slice g / 32, lane g % 32, entry j at sliceOff + 32 j + lane
+    const int64_t base = sliceOff[g >> 5] + (g & 31);
+    const int glen = rowLen[g];
+    for (int64_t t = a; t < b; t++) {
+      const int c = idx[t];
+      const int kc = (c >= 0 && c < n) ? iperm[c] : -1;
+      const int64_t q = kc >= 0 ? find_sorted(patIdx, p0, len, 1, kc) : -1;
+      if (q < 0) { atomicAdd(cnt + UPD_NEU_OUTSIDE, 1ull); continue; }
+      if (atomicOr(hits + q, 2) & 2) { atomicAdd(cnt + UPD_NEU_DUP, 1ull); continue; }
+      const int64_t sl = find_sorted(col, base, glen, 32, gidx[kc]);
+      if (sl < 0) { atomicAdd(cnt + UPD_NEU_NOT_IN_A, 1ull); continue; }
+      neu[q] = val[t];
+      slot[q] = sl;
+      cover[sl] = 1;
+    }
+  }
+}
+__global__ void k_update_cover(int n, const int64_t* __restrict__ sliceOff, const int* __restrict__ rowLen,
+                               const unsigned char* __restrict__ cover, unsigned long long* cnt) {
+  for (int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; g < n; g += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t base = sliceOff[g >> 5] + (g & 31);
+    int miss = 0;
+    for (int j = 0; j < rowLen[g]; j++) miss += cover[base + 32 * (int64_t)j] == 0;
+    if (miss) atomicAdd(cnt, (unsigned long long)miss);
+  }
+}
+__global__ void __launch_bounds__(256) k_update_absmax(int64_t nnz, const double* __restrict__ v, unsigned long long* out) {
+  __shared__ unsigned long long sh[8];
+  unsigned long long m = 0;  // bit patterns of non-negative doubles order like the values
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < nnz; i += (int64_t)gridDim.x * blockDim.x) {
+    const double a = fabs(v[i]);
+    if (a == a) m = max(m, (unsigned long long)__double_as_longlong(a));
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < (int)(blockDim.x >> 5); w++) m = max(m, sh[w]);
+    atomicMax(out, m);
+  }
+}
+__global__ void k_update_sell_add(int64_t nnz, const int64_t* __restrict__ slot, const double* __restrict__ neu, double* __restrict__ val) {
+  for (int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; q < nnz; q += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t s = slot[q];
+    if (s >= 0) val[s] += neu[q];
+  }
+}
+__global__ void k_update_robin(int n, const int64_t* __restrict__ ptr, const int* __restrict__ idx, const double* __restrict__ d,
+                               const double* __restrict__ dir, const double* __restrict__ neu, double optim, double* __restrict__ rob) {
+  for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) {
+    const bool shared = d[k] < 1.;  // d = 1 / multiplicity
+    for (int64_t q = ptr[k]; q < ptr[k + 1]; q++)  // (rounded product, then sum: the host's v += optim * vNeu, no FMA)
+      rob[q] = (shared && d[idx[q]] < 1.) ? __dadd_rn(dir[q], __dmul_rn(optim, neu[q])) : dir[q];
+  }
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -423,9 +528,12 @@ void SellMatrix::build(const CsrHost& a, cudaStream_t st) {
       }
     }
   }
+  std::vector<int> len(n);
+  for (int r = 0; r < n; r++) len[r] = (int)(a.ptr[r + 1] - a.ptr[r]);
   sliceOff.upload(off, st);
   col.upload(c, st);
   val.upload(v, st);
+  rowLen.upload(len, st);
   CUDA_CHECK(::geneo::sync_stream(st));
 }
 
@@ -586,6 +694,40 @@ void vals_axpby(int64_t nnz, const double* a, double tau, const double* b, doubl
 void csr_sum_all(int64_t nnz, const double* val, double* out, cudaStream_t st) {
   CUDA_CHECK(cudaMemsetAsync(out, 0, sizeof(double), st));
   k_sum_all<<<GENEO_TICK(grid_for(nnz, 256, 4)), 256, 0, st>>>(nnz, val, out);
+}
+
+void update_nodes(int n, const int* perm, const int* gidx, const int* nodes, int* iperm, unsigned long long* cnt, cudaStream_t st) {
+  k_update_nodes<<<GENEO_TICK(grid_for(n, 256)), 256, 0, st>>>(n, perm, gidx, nodes, iperm, cnt);
+  CUDA_CHECK(cudaGetLastError());
+}
+void update_locate_dir(int n, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, const int* iperm,
+                       const int64_t* patPtr, const int* patIdx, int* hits, double* dir, unsigned long long* cnt, cudaStream_t st) {
+  k_update_locate_dir<<<GENEO_TICK(grid_for(n, 256)), 256, 0, st>>>(n, nnz, ptr, idx, val, iperm, patPtr, patIdx, hits, dir, cnt);
+  CUDA_CHECK(cudaGetLastError());
+}
+void update_locate_neu(int n, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, const int* iperm, const int* gidx,
+                       const int64_t* patPtr, const int* patIdx, int* hits, const SellMatrix& A, double* neu, int64_t* slot,
+                       unsigned char* cover, unsigned long long* cnt, cudaStream_t st) {
+  k_update_locate_neu<<<GENEO_TICK(grid_for(n, 256)), 256, 0, st>>>(n, nnz, ptr, idx, val, iperm, gidx, patPtr, patIdx, hits,
+                                                                    A.sliceOff.p, A.col.p, A.rowLen.p, neu, slot, cover, cnt);
+  CUDA_CHECK(cudaGetLastError());
+}
+void update_cover_check(const SellMatrix& A, const unsigned char* cover, unsigned long long* cnt, cudaStream_t st) {
+  k_update_cover<<<GENEO_TICK(grid_for(A.n, 256)), 256, 0, st>>>(A.n, A.sliceOff.p, A.rowLen.p, cover, cnt);
+  CUDA_CHECK(cudaGetLastError());
+}
+void update_absmax(int64_t nnz, const double* v, unsigned long long* out, cudaStream_t st) {
+  k_update_absmax<<<GENEO_TICK(grid_for(nnz, 256, 4)), 256, 0, st>>>(nnz, v, out);
+  CUDA_CHECK(cudaGetLastError());
+}
+void update_sell_add(int64_t nnz, const int64_t* slot, const double* neu, SellMatrix& A, cudaStream_t st) {
+  k_update_sell_add<<<GENEO_TICK(grid_for(nnz, 256)), 256, 0, st>>>(nnz, slot, neu, A.val.p);
+  CUDA_CHECK(cudaGetLastError());
+}
+void update_robin(int n, const int64_t* ptr, const int* idx, const double* d, const double* dir, const double* neu, double optim,
+                  double* rob, cudaStream_t st) {
+  k_update_robin<<<GENEO_TICK(grid_for(n, 256)), 256, 0, st>>>(n, ptr, idx, d, dir, neu, optim, rob);
+  CUDA_CHECK(cudaGetLastError());
 }
 
 }  // namespace geneo

@@ -15,6 +15,7 @@ struct SellMatrix {
   DevBuf<int64_t> sliceOff;  // [nslices+1]
   DevBuf<int> col;
   DevBuf<double> val;
+  DevBuf<int> rowLen;     // [n] true entries of every row (padding carries column = row and value 0: not searchable)
   void build(const CsrHost& a, cudaStream_t st);
   // algorithmic bytes of one SpMV (CSR formula of SURVEY.md 8d): nnz*12 + (n+1)*4 + 16*n
   double algo_bytes() const { return (double)nnz * 12. + ((double)n + 1.) * 4. + 16. * (double)n; }
@@ -79,5 +80,32 @@ void rows_scale(int n, int ld, const double* d, double* Z, cudaStream_t st);    
 void csr_scale_sym(int n, const int64_t* ptr, const int* idx, const double* val, const double* d, double* out, cudaStream_t st);
 void vals_axpby(int64_t nnz, const double* a, double tau, const double* b, double* out, cudaStream_t st);  // out = a - tau b
 void csr_sum_all(int64_t nnz, const double* val, double* out, cudaStream_t st);               // out[0] = sum(val) (zeroed by the call)
+
+// ---- same-pattern value update (GeneoPC::check_values / commit_values) -----------------------------------------------
+// One thread per input row.  The locate kernels write no value the preconditioner uses: the located values land in fresh
+// buffers and every mismatch is counted into cnt[UPD_*] (one set of counters per subdomain, read back once).  The
+// duplicate counters are a defensive check: the library's own inputs cannot carry a duplicate column (the pre-decomposed
+// input refuses one when the problem is built, the decomposition never makes one).
+enum { UPD_NODES, UPD_DIR_ROW, UPD_DIR_OUTSIDE, UPD_DIR_DUP, UPD_NEU_OUTSIDE, UPD_NEU_DUP, UPD_NEU_NOT_IN_A, UPD_ANORM, UPD_SLOTS };
+// iperm[perm[k]] = k; cnt[UPD_NODES] += (gidx[k] != nodes[perm[k]])
+void update_nodes(int n, const int* perm, const int* gidx, const int* nodes, int* iperm, unsigned long long* cnt, cudaStream_t st);
+// input CSR (ptr, idx, val) of A_dir, natural order -> dir[q] on the permuted pattern (patPtr, patIdx; rows sorted by column).
+// Every row must have the stored row's length; hits (zeroed by the caller) bit 0 marks a filled q (duplicates).
+void update_locate_dir(int n, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, const int* iperm,
+                       const int64_t* patPtr, const int* patIdx, int* hits, double* dir, unsigned long long* cnt, cudaStream_t st);
+// input CSR of A_neu -> neu[q] (zeroed by the caller) on the same pattern and, per q, the slot of the operator A it adds to
+// (row gidx[k], column gidx[kc]; slot[q] stays -1 off the A_neu pattern); cover[slot] = 1 marks the operator's entries reached
+void update_locate_neu(int n, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, const int* iperm, const int* gidx,
+                       const int64_t* patPtr, const int* patIdx, int* hits, const SellMatrix& A, double* neu, int64_t* slot,
+                       unsigned char* cover, unsigned long long* cnt, cudaStream_t st);
+// *cnt += number of true entries of A that no A_neu entry reached
+void update_cover_check(const SellMatrix& A, const unsigned char* cover, unsigned long long* cnt, cudaStream_t st);
+// *out = bits of max |v| (atomicMax on the bit pattern: exact, order-free; NaN ignored like std::max(amax, NaN) does)
+void update_absmax(int64_t nnz, const double* v, unsigned long long* out, cudaStream_t st);
+// A.val[slot[q]] += neu[q] where slot[q] >= 0 (a subdomain reaches every slot at most once: no atomics)
+void update_sell_add(int64_t nnz, const int64_t* slot, const double* neu, SellMatrix& A, cudaStream_t st);
+// Robin values (createRobinMatrix): rob[q] = dir[q] + optim * neu[q] where row and column are shared (d < 1), dir[q] elsewhere
+void update_robin(int n, const int64_t* ptr, const int* idx, const double* d, const double* dir, const double* neu, double optim,
+                  double* rob, cudaStream_t st);
 
 }  // namespace geneo
