@@ -169,7 +169,8 @@ class GeneoPC:
     TIMER_NAMES = ["lvl1SetupMinv", "lvl2SetupTauLoc", "lvl2SetupTauSyl", "lvl2SetupTauEig", "lvl2SetupGammaLoc",
                    "lvl2SetupGammaSyl", "lvl2SetupGammaEig", "lvl2SetupSyl", "lvl2SetupEig", "lvl2SetupZ", "lvl2SetupE",
                    "lvl1Apply", "lvl1ApplyScatter", "lvl1ApplyMinv", "lvl1ApplyGather", "lvl1ApplyPrjFS", "lvl2Apply",
-                   "lvl2ApplyZt", "lvl2ApplyEinv", "lvl2ApplyZ", "symbolic", "operator", "setup", "upload", "numeric"]
+                   "lvl2ApplyZt", "lvl2ApplyEinv", "lvl2ApplyZ", "symbolic", "operator", "setup", "upload", "numeric",
+                   "update_layout"]
 
     def __init__(self, options=None):
         self.h = C.c_void_p()

@@ -385,11 +385,14 @@ int geneo_pc_refactor(geneo_pc_t pc) {
 int geneo_pc_update(geneo_pc_t pc, geneo_problem_t p) {
   ABI_TRY
   ABI_REQ(pc && pc->ready, "GenEO preconditioner without context");
-  ABI_REQ(p && p->decomposed, "GenEO preconditioner without a decomposed problem");
-  ABI_REQ(!pc->dist, "same-pattern update of a multi-GPU preconditioner (geneo_pc_setup_dist) is not supported: set it up again");
-  require_device();
   GeneoPC::PendingValues nv;
-  pc->pc.check_values(p->dec, nv);  // throws on any mismatch before a resident value changes: the PC stays as it was
+  if (pc->dist) {  // collective: a problem this rank cannot use is its vote against the update, not an early return
+    pc->pc.check_values_dist(p ? &p->mesh : nullptr, p && p->decomposed ? &p->dec : nullptr, nv);
+  } else {
+    ABI_REQ(p && p->decomposed, "GenEO preconditioner without a decomposed problem");
+    require_device();
+    pc->pc.check_values(p->dec, nv);  // throws on any mismatch before a resident value changes: the PC stays as it was
+  }
   pc->ready = false;                // from here on values and factors disagree until the numeric setup has completed
   pc->prob = p;
   pc->pc.commit_values(nv);
@@ -483,7 +486,8 @@ int geneo_pc_timers(geneo_pc_t pc, double* t, int cap) {
                       g.lvl2SetupSylTime, g.lvl2SetupEigTime, g.lvl2SetupZTime, g.lvl2SetupETime,   // 7-10
                       g.lvl1ApplyTime, g.lvl1ApplyScatterTime, g.lvl1ApplyMinvTime, g.lvl1ApplyGatherTime,  // 11-14
                       g.lvl1ApplyPrjFSTime, g.lvl2ApplyTime, g.lvl2ApplyZtTime, g.lvl2ApplyEinvTime, g.lvl2ApplyZTime,  // 15-19
-                      g.symbolicTime, g.operatorTime, g.setupTime, g.uploadTime, g.numericTime};   // 20-24
+                      g.symbolicTime, g.operatorTime, g.setupTime, g.uploadTime, g.numericTime,    // 20-24
+                      g.updateLayoutTime};                                                          // 25
   const int n = (int)(sizeof(v) / sizeof(v[0]));
   for (int i = 0; i < std::min(n, cap); i++) t[i] = v[i];
   ABI_CATCH

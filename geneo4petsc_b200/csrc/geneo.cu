@@ -729,7 +729,15 @@ void GeneoPC::setup(const Decomposition& dec, const RankLayout* layout, const vo
   nbPart = dec.nbPart;
   scal.alloc(1024);
   std::vector<const Subdomain*> mine;
+  distKeys = DistKeys();
   if (layout) {
+    distKeys.dist = true;
+    distKeys.rank = layout->rank;
+    distKeys.world = layout->world;
+    distKeys.subRank = layout->subRank;
+    distKeys.owned = layout->owned;
+    distKeys.ghost = layout->ghost;
+    distKeys.ghostPtr = layout->ghostPtr;
     nOwn = layout->nOwn();
     nLoc = nOwn + layout->nGhost();
     for (auto& S : dec.subs)
@@ -1118,10 +1126,13 @@ void GeneoPC::numeric_setup() {
 // gidx, d, the operator's SELL layout, lanes and workspaces.  Per subdomain the new CSR matrices go up through one staging
 // set sized for the largest subdomain and are located on the device in the setup's pattern; the values land in fresh
 // buffers (PendingValues), and the counters of every check are read back once.  Only commit_values() writes resident values.
-void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv) {
+// With a layout (multi-GPU) gidx is rank-local and the operator holds only the owned rows, assembled from the elements:
+// node ids are compared in the layout's local numbering, A_neu is not located in the operator, and the layout's owned rows
+// are checked against the operator's pattern and placed into nv.op instead.
+void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv, const RankLayout* layout) {
   require_device();
   const int P = (int)subs.size();
-  GENEO_CHECK(P > 0 && !comm.active(), "update: the preconditioner is not set up on one process");
+  GENEO_CHECK(P > 0 && (layout != nullptr) == distKeys.dist, "update: the preconditioner is not set up for this kind of update");
   auto fail = [](const std::string& m) { throw Error("geneo_b200: same-pattern update: " + m); };
   if (dec.nbPart != nbPart)
     fail("the problem has " + std::to_string(dec.nbPart) + " subdomains, the preconditioner was set up with " + std::to_string(nbPart));
@@ -1130,7 +1141,7 @@ void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv) {
   int nMax = 0;
   int64_t zMax = 0;
   for (int p = 0; p < P; p++) {
-    const Subdomain& S = dec.subs[p];
+    const Subdomain& S = dec.subs[subs[p].id];
     const SubdomainState& s = subs[p];
     const std::string sub = "subdomain " + std::to_string(s.id) + ": ";
     if (S.id != s.id || (int)S.nodes.size() != s.n) fail(sub + "the node set differs from the setup's (another partition?)");
@@ -1142,18 +1153,20 @@ void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv) {
     nMax = std::max(nMax, s.n);
     zMax = std::max(zMax, s.pat.nnz);
   }
+  if (layout) zMax = std::max<int64_t>(zMax, layout->A.nnz());  // the staging set carries the owned rows too
   CUDA_CHECK(::geneo::sync_stream(st));
-  DevBuf<int64_t> dPtr((size_t)nMax + 1);
+  DevBuf<int64_t> dPtr((size_t)std::max(nMax, layout ? nOwn : 0) + 1);
   DevBuf<int> dIdx((size_t)zMax), dNodes((size_t)nMax), dIperm((size_t)nMax), hits((size_t)zMax);
   DevBuf<double> dVal((size_t)zMax);
-  DevBuf<unsigned long long> cnt((size_t)P * UPD_SLOTS + 1);  // + the operator entries no A_neu reached
-  DevBuf<unsigned char> cover((size_t)A.stored);
+  DevBuf<unsigned long long> cnt((size_t)P * UPD_SLOTS + 1);  // + the operator entries no A_neu reached / owned rows that differ
+  DevBuf<unsigned char> cover(layout ? 0 : (size_t)A.stored);
   cnt.zero(st);
   cover.zero(st);
   nv.subs.clear();
   nv.subs.resize(P);
+  std::vector<int> local;
   for (int p = 0; p < P; p++) {
-    const Subdomain& S = dec.subs[p];
+    const Subdomain& S = dec.subs[subs[p].id];
     SubdomainState& s = subs[p];
     const int n = s.n;
     const int64_t nnz = s.pat.nnz, nnzNeu = s.neuNnz;
@@ -1161,11 +1174,19 @@ void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv) {
     PendingValues::Sub& w = nv.subs[p];
     w.dir.alloc((size_t)nnz);
     w.neu.alloc((size_t)nnz);
-    w.slot.alloc((size_t)nnz);
     w.neu.zero(st);
-    CUDA_CHECK(cudaMemsetAsync(w.slot.p, 0xff, (size_t)nnz * sizeof(int64_t), st));  // -1: off the A_neu pattern
+    if (!layout) {
+      w.slot.alloc((size_t)nnz);
+      CUDA_CHECK(cudaMemsetAsync(w.slot.p, 0xff, (size_t)nnz * sizeof(int64_t), st));  // -1: off the A_neu pattern
+    }
     CUDA_CHECK(cudaMemsetAsync(hits.p, 0, (size_t)nnz * sizeof(int), st));
-    dNodes.upload(S.nodes.data(), (size_t)n, st);
+    if (layout) {  // gidx holds local indices: compare against the new layout's numbering of the node ids
+      local.resize((size_t)n);
+      for (int l = 0; l < n; l++) local[l] = layout->local(S.nodes[l]);
+      dNodes.upload(local.data(), (size_t)n, st);
+    } else {
+      dNodes.upload(S.nodes.data(), (size_t)n, st);
+    }
     update_nodes(n, s.plan->dPerm.p, s.gidx.p, dNodes.p, dIperm.p, c, st);
     dPtr.upload(S.aDir.ptr.data(), (size_t)n + 1, st);
     dIdx.upload(S.aDir.idx.data(), (size_t)nnz, st);
@@ -1178,7 +1199,18 @@ void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv) {
     update_locate_neu(n, nnzNeu, dPtr.p, dIdx.p, dVal.p, dIperm.p, s.gidx.p, s.pat.ptr.p, s.pat.idx.p, hits.p, A, w.neu.p, w.slot.p,
                       cover.p, c, st);
   }
-  update_cover_check(A, cover.p, cnt.p + (size_t)P * UPD_SLOTS, st);
+  if (layout) {
+    const CsrHost& R = layout->A;
+    GENEO_CHECK(R.n == nOwn, "update: the rebuilt layout has another number of owned rows");
+    nv.op.alloc(A.val.n);
+    nv.op.zero(st);  // the padding of the SELL layout
+    dPtr.upload(R.ptr.data(), (size_t)R.n + 1, st);
+    dIdx.upload(R.idx.data(), (size_t)R.nnz(), st);
+    dVal.upload(R.val.data(), (size_t)R.nnz(), st);
+    update_owned_rows(A, R.nnz(), dPtr.p, dIdx.p, dVal.p, nv.op.p, cnt.p + (size_t)P * UPD_SLOTS, st);
+  } else {
+    update_cover_check(A, cover.p, cnt.p + (size_t)P * UPD_SLOTS, st);
+  }
   const std::vector<unsigned long long> h = cnt.to_host(st);  // the only read-back
   static const char* what[UPD_ANORM] = {
       "node ids differ from the setup's", "A_dir rows whose length differs from the setup's", "A_dir entries outside the setup's pattern",
@@ -1188,23 +1220,56 @@ void GeneoPC::check_values(const Decomposition& dec, PendingValues& nv) {
     for (int e = 0; e < UPD_ANORM; e++)
       if (h[(size_t)p * UPD_SLOTS + e])
         fail("subdomain " + std::to_string(subs[p].id) + ": " + std::to_string(h[(size_t)p * UPD_SLOTS + e]) + " " + what[e]);
-  if (h[(size_t)P * UPD_SLOTS]) fail(std::to_string(h[(size_t)P * UPD_SLOTS]) + " entries of the operator are in no subdomain's A_neu");
+  if (h[(size_t)P * UPD_SLOTS])
+    fail(std::to_string(h[(size_t)P * UPD_SLOTS]) +
+         (layout ? " owned rows of the operator differ from the setup's pattern" : " entries of the operator are in no subdomain's A_neu"));
   for (int p = 0; p < P; p++) memcpy(&nv.subs[p].anorm, &h[(size_t)p * UPD_SLOTS + UPD_ANORM], sizeof(double));
 }
 
-// The checked values replace the resident ones.  Operator: zero, then + A_neu,p subdomain by subdomain in ascending order --
-// the host merge of setup() sums 0 + a_1 + a_2 ... in the same order, so A, mult() and everything downstream match a fresh
-// setup bit for bit.
+void GeneoPC::check_values_dist(const Mesh* mesh, const Decomposition* dec, PendingValues& nv) {
+  GENEO_CHECK(distKeys.dist, "update: the preconditioner is not set up on several GPUs");
+  const DistKeys& K = distKeys;
+  std::string err;
+  try {
+    auto fail = [](const std::string& m) { throw Error("geneo_b200: same-pattern update: " + m); };
+    if (!mesh || !dec) fail("this rank has no decomposed problem");
+    if (dec->nbPart != nbPart)
+      fail("the problem has " + std::to_string(dec->nbPart) + " subdomains, the preconditioner was set up with " + std::to_string(nbPart));
+    const double t0 = now_s();
+    RankLayout L;
+    build_rank_layout(*mesh, *dec, K.subRank, K.rank, K.world, L);
+    updateLayoutTime = now_s() - t0;
+    if (L.owned != K.owned || L.ghost != K.ghost || L.ghostPtr != K.ghostPtr)
+      fail("the rank's owned / ghost nodes differ from the setup's (another partition or sub_rank?)");
+    check_values(*dec, nv, &L);
+  } catch (std::exception& e) {
+    err = e.what();
+  }
+  std::vector<double> vote((size_t)K.world, 0.);  // 1 where a rank rejects the update
+  vote[K.rank] = err.empty() ? 0. : 1.;
+  comm.allreduce_sum_host(vote.data(), K.world, st);
+  if (!err.empty()) throw Error(err);
+  for (int q = 0; q < K.world; q++)
+    if (vote[q] > 0.5)
+      throw Error("geneo_b200: same-pattern update rejected by rank " + std::to_string(q) +
+                  " (its own message gives the reason); the preconditioner is left as it was");
+}
+
+// The checked values replace the resident ones.  Operator, one process: zero, then + A_neu,p subdomain by subdomain in
+// ascending order -- the host merge of setup() sums 0 + a_1 + a_2 ... in the same order, so A, mult() and everything
+// downstream match a fresh setup bit for bit.  Multi-GPU: the owned rows placed by check_values (no sum) become A's values.
 void GeneoPC::commit_values(PendingValues& nv) {
   GENEO_CHECK(nv.subs.size() == subs.size(), "commit_values: the pending values do not belong to this preconditioner");
-  CUDA_CHECK(cudaMemsetAsync(A.val.p, 0, A.val.bytes(), st));
+  GENEO_CHECK(!distKeys.dist || nv.op.n == A.val.n, "commit_values: the pending operator does not belong to this preconditioner");
+  if (distKeys.dist) A.val = std::move(nv.op);
+  else CUDA_CHECK(cudaMemsetAsync(A.val.p, 0, A.val.bytes(), st));
   for (size_t p = 0; p < subs.size(); p++) {
     SubdomainState& s = subs[p];
     PendingValues::Sub& w = nv.subs[p];
     s.anorm = w.anorm;
     s.pat.val = std::move(w.dir);
     s.vNeu = std::move(w.neu);
-    update_sell_add(s.pat.nnz, w.slot.p, s.vNeu.p, A, st);
+    if (!distKeys.dist) update_sell_add(s.pat.nnz, w.slot.p, s.vNeu.p, A, st);
     if (opt.lvl1ORAS) {  // createRobinMatrix, as prepare_subdomain does it
       if ((int64_t)s.vRob.n != s.pat.nnz) s.vRob.alloc((size_t)s.pat.nnz);
       if (std::fabs(opt.optim) > DBL_EPSILON) update_robin(s.n, s.pat.ptr.p, s.pat.idx.p, s.d.p, s.pat.val.p, s.vNeu.p, opt.optim, s.vRob.p, st);

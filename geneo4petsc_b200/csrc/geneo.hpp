@@ -95,6 +95,7 @@ class GeneoPC {
   double lvl1ApplyTime = 0., lvl1ApplyScatterTime = 0., lvl1ApplyMinvTime = 0., lvl1ApplyGatherTime = 0.;
   double lvl1ApplyPrjFSTime = 0., lvl2ApplyTime = 0., lvl2ApplyZtTime = 0., lvl2ApplyEinvTime = 0., lvl2ApplyZTime = 0.;
   double symbolicTime = 0., operatorTime = 0., setupTime = 0., uploadTime = 0., numericTime = 0., orderingReuseTime = 0.;
+  double updateLayoutTime = 0.;  // last same-pattern update of a multi-GPU PC: host rebuild of the rank's layout
   int estimDimE = 0, realDimE = 0, nicolaides = 0;
   int64_t factorBytes = 0, factorNnz = 0, applyCount = 0;
   double factorFlops = 0.;
@@ -111,19 +112,35 @@ class GeneoPC {
   // layout->subRank[p] == rank are local, vectors are [owned | ghost] (RankLayout), comm holds the NCCL plumbing.
   void setup(const Decomposition& dec, const RankLayout* layout = nullptr, const void* ncclUid = nullptr);
   Comm comm;
+  // Multi-GPU setup (layout given): the rank's place and the layout's node lists, which a same-pattern update must reproduce
+  // for the local numbering, the halo send lists and comm to stay valid.  `dist` is false after a single-GPU setup.
+  struct DistKeys {
+    bool dist = false;
+    int rank = 0, world = 1;
+    std::vector<int> subRank, owned, ghost;
+    std::vector<int64_t> ghostPtr;
+  } distKeys;
   // Numeric half of the setup again (every factorization, eigen-solve, Z, E) on the matrices already resident in HBM:
   // PCSetUp with an unchanged non-zero pattern.  setup() = host analysis + uploads + numeric_setup().
   void numeric_setup();
-  // PCSetUp with SAME_NONZERO_PATTERN and new values (single process), in three steps: check_values() uploads the A_dir /
-  // A_neu values of `dec` -- same partition, node sets and patterns as the last setup() -- locates them in the resident
-  // pattern and checks them on the device without writing any resident value (on a mismatch it throws and the
-  // preconditioner is left as it was); commit_values() puts them in place (A_dir, A_neu, the Robin values, the operator,
-  // the pivot scale); numeric_setup() must follow before the next apply.
+  // PCSetUp with SAME_NONZERO_PATTERN and new values, in three steps: check_values() uploads the A_dir / A_neu values of
+  // `dec` -- same partition, node sets and patterns as the last setup() -- locates them in the resident pattern and checks
+  // them on the device without writing any resident value (on a mismatch it throws and the preconditioner is left as it
+  // was); commit_values() puts them in place (A_dir, A_neu, the Robin values, the operator, the pivot scale);
+  // numeric_setup() must follow before the next apply.
+  // On one process the operator is re-summed from the A_neu values.  On a multi-GPU PC (`layout`: the rank's layout rebuilt
+  // from the new problem) the operator's owned rows are the layout's, placed into a fresh value buffer (op).
   struct PendingValues {
     struct Sub { DevBuf<double> dir, neu; DevBuf<int64_t> slot; double anorm = 0.; };  // slot: operator entry of A_neu q, or -1
     std::vector<Sub> subs;
+    DevBuf<double> op;  // multi-GPU: the operator's new values, SELL layout of A
   };
-  void check_values(const Decomposition& dec, PendingValues& nv);
+  void check_values(const Decomposition& dec, PendingValues& nv, const RankLayout* layout = nullptr);
+  // Multi-GPU PC, collective: every rank passes its own problem (null when it has none, `dec` null when it is not
+  // decomposed).  Rebuilds the rank's layout from `mesh` / `dec` as setup's caller did (build_rank_layout), requires the
+  // setup's owned / ghost lists, then check_values().  Every rank's verdict goes into one vote: either all ranks return with their pending values or all throw
+  // (a rejecting rank with its own reason, the others naming it), so no rank commits while another one rejects.
+  void check_values_dist(const Mesh* mesh, const Decomposition* dec, PendingValues& nv);
   void commit_values(PendingValues& nv);
   void numeric_begin();
   void numeric_end();

@@ -444,14 +444,15 @@ __global__ void k_update_locate_neu(int n, int64_t nnz, const int64_t* __restric
     const int64_t a = ptr[r], b = ptr[r + 1], p0 = patPtr[k], len = patPtr[k + 1] - p0;
     if (a < 0 || b < a || b > nnz) { atomicAdd(cnt + UPD_NEU_OUTSIDE, 1ull); continue; }
     const int g = gidx[k];  // row of the operator: slice g / 32, lane g % 32, entry j at sliceOff + 32 j + lane
-    const int64_t base = sliceOff[g >> 5] + (g & 31);
-    const int glen = rowLen[g];
+    const int64_t base = slot ? sliceOff[g >> 5] + (g & 31) : 0;
+    const int glen = slot ? rowLen[g] : 0;
     for (int64_t t = a; t < b; t++) {
       const int c = idx[t];
       const int kc = (c >= 0 && c < n) ? iperm[c] : -1;
       const int64_t q = kc >= 0 ? find_sorted(patIdx, p0, len, 1, kc) : -1;
       if (q < 0) { atomicAdd(cnt + UPD_NEU_OUTSIDE, 1ull); continue; }
       if (atomicOr(hits + q, 2) & 2) { atomicAdd(cnt + UPD_NEU_DUP, 1ull); continue; }
+      if (!slot) { neu[q] = val[t]; continue; }  // no operator lookup (multi-GPU: the operator rows come from the layout)
       const int64_t sl = find_sorted(col, base, glen, 32, gidx[kc]);
       if (sl < 0) { atomicAdd(cnt + UPD_NEU_NOT_IN_A, 1ull); continue; }
       neu[q] = val[t];
@@ -467,6 +468,24 @@ __global__ void k_update_cover(int n, const int64_t* __restrict__ sliceOff, cons
     int miss = 0;
     for (int j = 0; j < rowLen[g]; j++) miss += cover[base + 32 * (int64_t)j] == 0;
     if (miss) atomicAdd(cnt, (unsigned long long)miss);
+  }
+}
+// one thread per owned row g: the input row (ptr, idx, val) must have the operator row's length and, position by position,
+// its columns (both sorted by local column); its values go to the same slots of `out`
+__global__ void k_update_owned_rows(int n, int64_t nnz, const int64_t* __restrict__ ptr, const int* __restrict__ idx,
+                                    const double* __restrict__ val, const int64_t* __restrict__ sliceOff, const int* __restrict__ col,
+                                    const int* __restrict__ rowLen, double* __restrict__ out, unsigned long long* cnt) {
+  for (int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; g < n; g += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t a = ptr[g], b = ptr[g + 1], base = sliceOff[g >> 5] + (g & 31);
+    const int len = rowLen[g];
+    if (a < 0 || b > nnz || b - a != len) { atomicAdd(cnt, 1ull); continue; }
+    bool same = true;
+    for (int j = 0; j < len; j++) {
+      const int64_t o = base + 32 * (int64_t)j;
+      same = same && idx[a + j] == col[o];
+      out[o] = val[a + j];
+    }
+    if (!same) atomicAdd(cnt, 1ull);
   }
 }
 __global__ void __launch_bounds__(256) k_update_absmax(int64_t nnz, const double* __restrict__ v, unsigned long long* out) {
@@ -714,6 +733,11 @@ void update_locate_neu(int n, int64_t nnz, const int64_t* ptr, const int* idx, c
 }
 void update_cover_check(const SellMatrix& A, const unsigned char* cover, unsigned long long* cnt, cudaStream_t st) {
   k_update_cover<<<GENEO_TICK(grid_for(A.n, 256)), 256, 0, st>>>(A.n, A.sliceOff.p, A.rowLen.p, cover, cnt);
+  CUDA_CHECK(cudaGetLastError());
+}
+void update_owned_rows(const SellMatrix& A, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, double* out,
+                       unsigned long long* cnt, cudaStream_t st) {
+  k_update_owned_rows<<<GENEO_TICK(grid_for(A.n, 256)), 256, 0, st>>>(A.n, nnz, ptr, idx, val, A.sliceOff.p, A.col.p, A.rowLen.p, out, cnt);
   CUDA_CHECK(cudaGetLastError());
 }
 void update_absmax(int64_t nnz, const double* v, unsigned long long* out, cudaStream_t st) {

@@ -94,12 +94,18 @@ void update_nodes(int n, const int* perm, const int* gidx, const int* nodes, int
 void update_locate_dir(int n, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, const int* iperm,
                        const int64_t* patPtr, const int* patIdx, int* hits, double* dir, unsigned long long* cnt, cudaStream_t st);
 // input CSR of A_neu -> neu[q] (zeroed by the caller) on the same pattern and, per q, the slot of the operator A it adds to
-// (row gidx[k], column gidx[kc]; slot[q] stays -1 off the A_neu pattern); cover[slot] = 1 marks the operator's entries reached
+// (row gidx[k], column gidx[kc]; slot[q] stays -1 off the A_neu pattern); cover[slot] = 1 marks the operator's entries reached.
+// slot == nullptr (multi-GPU, where gidx is rank-local and A holds only the owned rows): no operator lookup, cover unused.
 void update_locate_neu(int n, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, const int* iperm, const int* gidx,
                        const int64_t* patPtr, const int* patIdx, int* hits, const SellMatrix& A, double* neu, int64_t* slot,
                        unsigned char* cover, unsigned long long* cnt, cudaStream_t st);
 // *cnt += number of true entries of A that no A_neu entry reached
 void update_cover_check(const SellMatrix& A, const unsigned char* cover, unsigned long long* cnt, cudaStream_t st);
+// Multi-GPU: the owned rows (ptr, idx, val: CSR, A.n rows, local columns sorted) must have A's row lengths and columns
+// position by position; their values go to the same slots of `out` (A.val's layout, padding zeroed by the caller).
+// *cnt += rows that differ.
+void update_owned_rows(const SellMatrix& A, int64_t nnz, const int64_t* ptr, const int* idx, const double* val, double* out,
+                       unsigned long long* cnt, cudaStream_t st);
 // *out = bits of max |v| (atomicMax on the bit pattern: exact, order-free; NaN ignored like std::max(amax, NaN) does)
 void update_absmax(int64_t nnz, const double* v, unsigned long long* out, cudaStream_t st);
 // A.val[slot[q]] += neu[q] where slot[q] >= 0 (a subdomain reaches every slot at most once: no atomics)

@@ -89,18 +89,26 @@ int geneo_pc_refactor(geneo_pc_t pc);
 /* PCSetUp again after the operator's VALUES changed and its pattern did not (PETSc's SAME_NONZERO_PATTERN: time steps
  * with a new dt, Newton steps, coefficient updates), re-entering setUpGenEOPC (src/geneo.cpp:1672-1843) without its
  * pattern work: the ordering, the symbolic analysis, the operator's layout and the uploaded plans of the last
- * geneo_pc_setup are kept; the new A_neu / A_dir values are uploaded, placed on the device, and the numeric setup (every
- * factorization, eigen-solve, Z and E) runs.  The PC is then what a fresh geneo_pc_setup(pc, p) would give.
+ * geneo_pc_setup / geneo_pc_setup_dist are kept; the new A_neu / A_dir values are uploaded, placed on the device, and the
+ * numeric setup (every factorization, eigen-solve, Z and E) runs.  The PC is then what a fresh setup on p would give.
  * p must be decomposed with the same nbPart as the last setup, every subdomain with the same node set and the same A_neu
- * and A_dir patterns; only the values may differ.  Fails with a message when the PC is not set up, p is not decomposed,
- * or the PC was set up with geneo_pc_setup_dist (not supported).  What is checked of the input: the partition and every
- * node set exactly; A_dir exactly (row by row: same length, every entry in the setup's pattern, none twice); A_neu by its
- * number of entries, each inside its row of the setup's A_dir pattern and in the operator's pattern, none twice, and the
- * A_neu of all subdomains together reaching every entry of the operator.  An A_neu entry moved within those bounds is
- * accepted, and the result is then still exactly what a fresh geneo_pc_setup on p builds (same operator layout, same
- * values).  All checks run before any resident value is overwritten: after a rejected update the PC still holds the
- * previous preconditioner.  If the numeric setup itself fails (e.g. -geneo_chk finds the
- * new A_dir not SPD), the PC is left without context until the next successful setup or update. */
+ * and A_dir patterns; only the values may differ.  Fails with a message when the PC is not set up or p is not decomposed.
+ * What is checked of the input: the partition and every node set exactly; A_dir exactly (row by row: same length, every
+ * entry in the setup's pattern, none twice); A_neu by its number of entries, each inside its row of the setup's A_dir
+ * pattern, none twice.  On one process each A_neu entry must also lie in the operator's pattern and the A_neu of all
+ * subdomains together must reach every entry of the operator; an A_neu entry moved within those bounds is accepted, and
+ * the result is then still exactly what a fresh geneo_pc_setup on p builds (same operator layout, same values).
+ * On a PC set up with geneo_pc_setup_dist the call is COLLECTIVE: every rank calls it with its own problem, built the way
+ * the setup's was (geneo_problem_generate_boxed + geneo_problem_decompose_owned, or the same METIS grouping) from the same
+ * partition and sub_rank.  The operator's owned rows are re-assembled from the rank's mesh by the layout code of
+ * geneo_layout_create; the rank's owned and ghost node lists must come out as at the setup (so the halo plan and the NCCL
+ * communicator stay), and every owned row must have the operator's pattern.  The operator, A_dir, A_neu and the Robin
+ * values are then bit for bit those of a fresh geneo_pc_setup_dist on the new problems.  All ranks vote on the checks:
+ * either every rank updates or every rank fails, a rank whose input was rejected with its own reason, the others with a
+ * message naming that rank.
+ * All checks run before any resident value is overwritten: after a rejected update the PC still holds the previous
+ * preconditioner.  If the numeric setup itself fails (e.g. -geneo_chk finds the new A_dir not SPD), the PC is left
+ * without context until the next successful setup or update. */
 int geneo_pc_update(geneo_pc_t pc, geneo_problem_t p);
 /* With -geneo_kernel_timing: CUDA-event time (ms) and launch count of the level-1 solve kernel since the last call. */
 int geneo_pc_kernel_time(geneo_pc_t pc, double* ms, int64_t* launches);
