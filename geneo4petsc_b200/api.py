@@ -316,7 +316,44 @@ class GeneoPC:
         return dict(x=x, its=int(out[0]), reason=int(out[1]), reason_name=KSP_REASONS.get(int(out[1]), "?"),
                     rnorm=rn.value, history=hist[: int(out[2])].copy())
 
+    def apply_block(self, X):
+        """PCMatApply: Y = M^-1 X for the k columns of X, shape (n, k) (or (n,)); 8 columns per pass over the factors."""
+        X = np.asarray(X, dtype=np.float64)
+        Xf = np.asfortranarray(X[:, None] if X.ndim == 1 else X)
+        Y = np.zeros(Xf.shape, order="F")
+        _chk(lib.geneo_pc_apply_block(self.h, C.c_int(Xf.shape[1]), _p(Xf, _f64p), C.c_int64(Xf.shape[0]), _p(Y, _f64p),
+                                      C.c_int64(Y.shape[0])))
+        return Y.reshape(X.shape)
+
+    def ksp_solve_block(self, B, ksp="cg", rtol=1e-5, atol=1e-50, dtol=1e5, max_it=10000):
+        """KSPMatSolve with lock-step CG on the k columns of B, shape (n, k): each column as ksp_solve(B[:, j], "cg")."""
+        B = np.asarray(B, dtype=np.float64)
+        Bf = np.asfortranarray(B[:, None] if B.ndim == 1 else B)
+        k = Bf.shape[1]
+        X = np.zeros(Bf.shape, order="F")
+        out, rn = np.zeros(2 * max(k, 1), dtype=np.int64), np.zeros(max(k, 1))
+        _chk(lib.geneo_ksp_solve_block(self.h, (ksp or "").encode(), C.c_int(k), _p(Bf, _f64p), C.c_int64(Bf.shape[0]),
+                                       _p(X, _f64p), C.c_int64(X.shape[0]), C.c_double(rtol), C.c_double(atol), C.c_double(dtol),
+                                       C.c_int(max_it), _p(out, _i64p), _p(rn, _f64p)))
+        return dict(x=X.reshape(B.shape), **self._block_result(out, rn, k))
+
+    @staticmethod
+    def _block_result(out, rn, k):
+        its, reason = out[0:2 * k:2].astype(int), out[1:2 * k:2].astype(int)
+        return dict(its=its, reason=reason, reason_name=[KSP_REASONS.get(int(r), "?") for r in reason], rnorm=rn[:k].copy())
+
     # device-pointer entry points (torch tensors' data_ptr())
+    def apply_block_device(self, dx_ptr, dy_ptr, k, ldx, ldy):
+        _chk(lib.geneo_pc_apply_block_device(self.h, C.c_int(k), C.c_void_p(dx_ptr), C.c_int64(ldx), C.c_void_p(dy_ptr),
+                                             C.c_int64(ldy)))
+
+    def ksp_solve_block_device(self, db_ptr, dx_ptr, k, ldb, ldx, ksp="cg", rtol=1e-5, atol=1e-50, dtol=1e5, max_it=10000):
+        out, rn = np.zeros(2 * max(k, 1), dtype=np.int64), np.zeros(max(k, 1))
+        _chk(lib.geneo_ksp_solve_block_device(self.h, (ksp or "").encode(), C.c_int(k), C.c_void_p(db_ptr), C.c_int64(ldb),
+                                              C.c_void_p(dx_ptr), C.c_int64(ldx), C.c_double(rtol), C.c_double(atol),
+                                              C.c_double(dtol), C.c_int(max_it), _p(out, _i64p), _p(rn, _f64p)))
+        return self._block_result(out, rn, k)
+
     def apply_device(self, dx_ptr, dy_ptr):
         _chk(lib.geneo_pc_apply_device(self.h, C.c_void_p(dx_ptr), C.c_void_p(dy_ptr)))
 

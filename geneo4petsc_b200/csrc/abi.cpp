@@ -453,6 +453,54 @@ int geneo_pc_apply_q_device(geneo_pc_t pc, const double* dx, double* dy) {
   pc->pc.applyQ(dx, dy);
   ABI_CATCH
 }
+// ---- blocks of right-hand sides ----------------------------------------------------------------------------------------
+// k and ksp are checked before the context, ld once the vector length is known
+#define BLOCK_REQ(pc, k, a, b, ld1, ld2)                                                                          \
+  ABI_REQ((k) >= 1, "block of right-hand sides: k must be at least 1");                                       \
+  ABI_REQ(pc && pc->ready && (a) && (b), "GenEO preconditioner without context");                            \
+  ABI_REQ((ld1) >= pc->pc.nLoc && (ld2) >= pc->pc.nLoc, "block of right-hand sides: leading dimension below the vector length")
+static void block_ksp_check(const char* ksp) {
+  const std::string k(ksp ? ksp : "(null)");
+  if (k != "cg") throw Error("geneo_b200: block solve: unsupported -ksp_type " + k + " (cg only; no block GMRES)");
+}
+static void block_report(const std::vector<KspResult>& r, int64_t* out, double* rnorm) {
+  for (size_t j = 0; j < r.size(); j++) {
+    if (out) { out[2 * j] = r[j].its; out[2 * j + 1] = r[j].reason; }
+    if (rnorm) rnorm[j] = r[j].rnorm;
+  }
+}
+// host column-major blocks go through the device 8 columns at a time: what = 0 apply, 1 CG solve
+static void stage_block(geneo_pc_t pc, int what, int k, const double* X, int64_t ldx, double* Y, int64_t ldy, double rtol,
+                        double atol, double dtol, int maxIt, int64_t* out, double* rnorm) {
+  GeneoPC& g = pc->pc;
+  const size_t n = (size_t)g.nLoc;
+  DevBuf<double> dx(n * 8), dy(n * 8);
+  for (int j0 = 0; j0 < k; j0 += 8) {
+    const int nc = std::min(8, k - j0);
+    for (int c = 0; c < nc; c++) h2d_staged(dx.p + c * n, X + (size_t)(j0 + c) * ldx, n * sizeof(double), g.st);
+    g_h2d_bytes += nc * n * sizeof(double);
+    if (what == 0) g.apply_block(nc, dx.p, (int64_t)n, dy.p, (int64_t)n);
+    else block_report(g.solve_cg_block(nc, dx.p, (int64_t)n, dy.p, (int64_t)n, rtol, atol, dtol, maxIt), out ? out + 2 * j0 : nullptr,
+                      rnorm ? rnorm + j0 : nullptr);
+    for (int c = 0; c < nc; c++)
+      CUDA_CHECK(cudaMemcpyAsync(Y + (size_t)(j0 + c) * ldy, dy.p + c * n, n * sizeof(double), cudaMemcpyDeviceToHost, g.st));
+    g_d2h_bytes += nc * n * sizeof(double);
+    CUDA_CHECK(::geneo::sync_stream(g.st));
+  }
+}
+int geneo_pc_apply_block(geneo_pc_t pc, int k, const double* X, int64_t ldx, double* Y, int64_t ldy) {
+  ABI_TRY
+  BLOCK_REQ(pc, k, X, Y, ldx, ldy);
+  stage_block(pc, 0, k, X, ldx, Y, ldy, 0., 0., 0., 0, nullptr, nullptr);
+  ABI_CATCH
+}
+int geneo_pc_apply_block_device(geneo_pc_t pc, int k, const double* dX, int64_t ldx, double* dY, int64_t ldy) {
+  ABI_TRY
+  BLOCK_REQ(pc, k, dX, dY, ldx, ldy);
+  pc->pc.apply_block(k, dX, ldx, dY, ldy);
+  ABI_CATCH
+}
+
 int geneo_pc_name(geneo_pc_t pc, char* buf, int cap) {
   ABI_TRY
   ABI_REQ(pc && buf && cap > 0, "null argument");
@@ -602,6 +650,22 @@ int geneo_ksp_solve(geneo_pc_t pc, const char* ksp, const double* b, double* x, 
   db.upload(b, g.nLoc, g.st);
   ksp_run(pc, ksp, db.p, dx.p, rtol, atol, dtol, maxIt, restart, out, rnorm, history, histCap);
   dx.download(x, g.nLoc, g.st);
+  ABI_CATCH
+}
+int geneo_ksp_solve_block(geneo_pc_t pc, const char* ksp, int k, const double* B, int64_t ldb, double* X, int64_t ldx,
+                          double rtol, double atol, double dtol, int maxIt, int64_t* out, double* rnorm) {
+  ABI_TRY
+  block_ksp_check(ksp);
+  BLOCK_REQ(pc, k, B, X, ldb, ldx);
+  stage_block(pc, 1, k, B, ldb, X, ldx, rtol, atol, dtol, maxIt, out, rnorm);
+  ABI_CATCH
+}
+int geneo_ksp_solve_block_device(geneo_pc_t pc, const char* ksp, int k, const double* dB, int64_t ldb, double* dX, int64_t ldx,
+                                 double rtol, double atol, double dtol, int maxIt, int64_t* out, double* rnorm) {
+  ABI_TRY
+  block_ksp_check(ksp);
+  BLOCK_REQ(pc, k, dB, dX, ldb, ldx);
+  block_report(pc->pc.solve_cg_block(k, dB, ldb, dX, ldx, rtol, atol, dtol, maxIt), out, rnorm);
   ABI_CATCH
 }
 const char* geneo_ksp_reason_name(int reason) { return ksp_reason_name(reason); }

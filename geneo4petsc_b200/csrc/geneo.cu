@@ -2110,6 +2110,90 @@ void GeneoPC::copy_einv(double* out) const {
     for (int j = 0; j < nE; j++) out[(size_t)i * nE + j] = h[(size_t)i * nEp + j];
 }
 
+// =====================================================================================================================
+// Block apply: the steps of applyQ / level1 / apply on row-major nLoc x 8 blocks, 8 columns per pass over the factors
+// =====================================================================================================================
+void GeneoPC::ensure_block() {
+  const size_t nb = (size_t)nLoc * 8, na = (size_t)nAll * 8, nw = (size_t)(nE + 7) / 8 * 8 * 8;
+  if (bIn.n != nb) { bIn.alloc(nb); bOut.alloc(nb); bT1.alloc(nb); bT2.alloc(nb); }
+  if (bXall.n != na) { bXall.alloc(na); bYall.alloc(na); }
+  if (bW.n != std::max<size_t>(nw, 8)) { bW.alloc(std::max<size_t>(nw, 8)); bW2.alloc(std::max<size_t>(nw, 8)); }
+}
+
+void GeneoPC::coarse8() {
+  const int nEp = (nE + 7) / 8 * 8;
+  bW.zero(st);
+  for (auto& s : subs) ts_gram(s.n, s.Z.p, s.nev, s.nev, bXall.p + (size_t)s.off * 8, 8, 8, bW.p + (size_t)s.zoff * 8, 8, st);
+  comm.allreduce_sum(bW.p, nE * 8, st);
+  ts_update(nE, Einv.p, nEp, nE, bW.p, 8, 8, bW2.p, 8, 1., 0., st);
+}
+
+void GeneoPC::applyQ8(double* x, double* y) {
+  comm.halo_forward(x, 8, st);
+  gather_rows8((int)nAll, gidxAll.p, x, bXall.p, st);
+  coarse8();
+  for (auto& s : subs)  // (beta 0: a subdomain without coarse vectors gets zero rows)
+    ts_update(s.n, s.Z.p, s.nev, s.nev, bW2.p + (size_t)s.zoff * 8, 8, 8, bYall.p + (size_t)s.off * 8, 8, 1., 0., st);
+  pull_sum8(nLoc, pullPtr.p, pullPos.p, bYall.p, y, st);
+  comm.halo_reverse_add(y, 8, st);
+}
+
+void GeneoPC::level1_8(double* x, double* y, bool addQ) {
+  comm.halo_forward(x, 8, st);
+  gather_rows8((int)nAll, gidxAll.p, x, bXall.p, st);
+  if (addQ) coarse8();
+  if (opt.lvl1RAS) rows_scale((int)nAll, 8, dAll.p, bXall.p, st);
+  forest.solve(bXall.p, bYall.p, 8, 0, 8, st);  // every local subdomain, 8 columns, in one launch of the 8-column kernel
+  for (auto& s : subs) {
+    double* ys = bYall.p + (size_t)s.off * 8;
+    if (opt.lvl1SRAS) rows_scale(s.n, 8, s.d.p, ys, st);
+    if (addQ && s.nev > 0) ts_update(s.n, s.Z.p, s.nev, s.nev, bW2.p + (size_t)s.zoff * 8, 8, 8, ys, 8, 1., 1., st);
+  }
+  pull_sum8(nLoc, pullPtr.p, pullPos.p, bYall.p, y, st);
+  comm.halo_reverse_add(y, 8, st);
+}
+
+void GeneoPC::mult8(double* x, double* y) {
+  comm.halo_forward(x, 8, st);
+  sell_spmm8(A, x, y, st);
+}
+void GeneoPC::mult_sub8(double* x, const double* b, double* y) {
+  mult8(x, y);
+  vec_axpby(A.n * 8, 1., b, -1., y, st);
+}
+
+void GeneoPC::apply8(double* x, double* y) {
+  const int n8 = nLoc * 8;
+  if (opt.lvl2 == 0) level1_8(x, y, false);
+  else if (!opt.hybrid) level1_8(x, y, true);
+  else if (!opt.effHybrid) {
+    applyQ8(x, bT1.p);                  // t1 = Q x
+    mult_sub8(bT1.p, x, bT2.p);         // t2 = x - A Q x
+    level1_8(bT2.p, y, false);          // y = t3
+    mult8(y, bT2.p);
+    applyQ8(bT2.p, bT2.p);              // t2 = Q A t3
+    vec_axpby(n8, -1., bT2.p, 1., y, st);  // y = (I - P) t3
+    vec_axpy(n8, 1., bT1.p, y, st);        // y += Q x
+  } else {
+    level1_8(x, y, false);
+    mult8(y, bT2.p);
+    applyQ8(bT2.p, bT2.p);
+    vec_axpby(n8, -1., bT2.p, 1., y, st);
+  }
+}
+
+void GeneoPC::apply_block(int k, const double* X, int64_t ldx, double* Y, int64_t ldy) {
+  GENEO_CHECK(k >= 1 && ldx >= nLoc && ldy >= nLoc, "block apply: k >= 1 and leading dimensions >= the vector length");
+  ensure_block();
+  for (int j0 = 0; j0 < k; j0 += 8) {
+    const int nc = std::min(8, k - j0);
+    pack_cols8(nLoc, nc, X + (size_t)j0 * ldx, ldx, bIn.p, st);
+    apply8(bIn.p, bOut.p);
+    unpack_cols8(nLoc, nc, bOut.p, Y + (size_t)j0 * ldy, ldy, st);
+  }
+  applyCount += k;
+}
+
 double GeneoPC::trisolve_algo_bytes() const {
   double b = 0.;
   for (auto& s : subs)
@@ -2286,6 +2370,106 @@ KspResult GeneoPC::solve_gmres(const double* b, double* x, double rtol, double a
   R.rnorm = res;
   R.reason = reason;
   return R;
+}
+
+std::vector<KspResult> GeneoPC::solve_cg_block(int k, const double* B, int64_t ldb, double* X, int64_t ldx, double rtol,
+                                               double atol, double dtol, int maxIt) {
+  GENEO_CHECK(k >= 1 && ldb >= nLoc && ldx >= nLoc, "block CG: k >= 1 and leading dimensions >= the vector length");
+  ensure_block();
+  std::vector<KspResult> res(k);
+  for (int j0 = 0; j0 < k; j0 += 8) {  // bIn = b, bOut = x of the chunk (apply8 leaves both alone)
+    const int nc = std::min(8, k - j0);
+    pack_cols8(nLoc, nc, B + (size_t)j0 * ldb, ldb, bIn.p, st);
+    if (opt.lvl2 >= 1 && opt.effHybrid) applyQ8(bIn.p, bOut.p);  // initial_guess: x0 = Q b, or 0
+    else bOut.zero(st);
+    cg8(bIn.p, bOut.p, (1u << nc) - 1u, rtol, atol, dtol, maxIt, res.data() + j0);
+    unpack_cols8(nLoc, nc, bOut.p, X + (size_t)j0 * ldx, ldx, st);
+  }
+  CUDA_CHECK(::geneo::sync_stream(st));
+  return res;
+}
+
+// solve_cg on the columns set in `active` (the others are zero padding), all of them in lock step: one block SpMV and one
+// block PC apply per iteration, the per-column dots in one pass and one host read-back each.  A column that stops is
+// frozen (its x and r are not written again) and keeps the its / reason / rnorm solve_cg would have returned.
+void GeneoPC::cg8(const double* b, double* x, unsigned active, double rtol, double atol, double dtol, int maxIt, KspResult* res) {
+  const int nc = 32 - __builtin_clz(active);
+  DevBuf<double> r((size_t)nLoc * 8), z((size_t)nLoc * 8), p((size_t)nLoc * 8), wv((size_t)nLoc * 8);
+  double h[16];
+  auto readback = [&](int cnt) {
+    comm.allreduce_sum(scal.p, cnt, st);
+    CUDA_CHECK(cudaMemcpyAsync(h, scal.p, cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_CHECK(::geneo::sync_stream(st));
+  };
+  mult_sub8(x, b, r.p);  // non-zero initial guess, as solve_cg
+  apply8(r.p, z.p);
+  dot_cols8(nOwn, z.p, r.p, z.p, scal.p, st);  // beta = z.r and ||z||^2
+  double zr[8], zz[8];
+  readback(16);
+  for (int c = 0; c < 8; c++) { zr[c] = h[c]; zz[c] = h[8 + c]; }
+  apply8(const_cast<double*>(b), wv.p);  // reference norm ||M^-1 b|| (b's ghost rows are refreshed, its owned rows kept)
+  applyCount += 2 * nc;
+  dot_cols8(nOwn, wv.p, wv.p, nullptr, scal.p, st);
+  readback(8);
+  ConvTest conv[8];
+  double beta[8], betaold[8];
+  for (int c = 0; c < 8; c++) {
+    beta[c] = 0.;
+    betaold[c] = 1.;
+    if (!((active >> c) & 1u)) continue;
+    KspResult& R = res[c];
+    const double dp = std::sqrt(zz[c]);
+    double sn = std::sqrt(h[c]);
+    if (sn == 0.) sn = dp;
+    conv[c].ttol = std::max(rtol * sn, atol); conv[c].rnorm0 = sn; conv[c].atol = atol; conv[c].dtol = dtol;
+    R.history.push_back(dp);
+    R.rnorm = dp;
+    R.reason = conv[c](dp);
+    if (R.reason) active &= ~(1u << c);
+    beta[c] = zr[c];
+  }
+  auto stop = [&](int c, int reason, int its) { res[c].reason = reason; res[c].its = its; active &= ~(1u << c); };
+  int i = 0;
+  while (active) {
+    for (int c = 0; c < 8; c++) {
+      if (!((active >> c) & 1u)) continue;
+      if (i >= maxIt) stop(c, KSP_DIVERGED_ITS, i);
+      else if (beta[c] == 0.) stop(c, KSP_CONVERGED_ATOL, i);
+      else if (i > 0 && beta[c] * betaold[c] < 0.) stop(c, KSP_DIVERGED_INDEFINITE_PC, i);
+    }
+    if (!active) break;
+    Coef8 cf{};
+    for (int c = 0; c < 8; c++) cf.v[c] = beta[c] / betaold[c];
+    if (i == 0) CUDA_CHECK(cudaMemcpyAsync(p.p, z.p, sizeof(double) * nLoc * 8, cudaMemcpyDeviceToDevice, st));
+    else aypx8(nLoc, cf, active, z.p, p.p, st);  // p = z + b p
+    mult8(p.p, wv.p);
+    dot_cols8(nOwn, p.p, wv.p, nullptr, scal.p, st);
+    readback(8);
+    for (int c = 0; c < 8; c++) {
+      if (!((active >> c) & 1u)) continue;
+      betaold[c] = beta[c];
+      if (h[c] <= 0.) stop(c, KSP_DIVERGED_INDEFINITE_MAT, i + 1);
+      else cf.v[c] = beta[c] / h[c];
+    }
+    cg_update8(nLoc, cf, active, p.p, wv.p, x, r.p, st);
+    if (!active) break;
+    apply8(r.p, z.p);
+    applyCount += __builtin_popcount(active);
+    dot_cols8(nOwn, z.p, r.p, z.p, scal.p, st);
+    readback(16);
+    for (int c = 0; c < 8; c++) {
+      if (!((active >> c) & 1u)) continue;
+      KspResult& R = res[c];
+      const double dp = std::sqrt(h[8 + c]);
+      R.history.push_back(dp);
+      R.rnorm = dp;
+      R.its = i + 1;
+      R.reason = conv[c](dp);
+      if (R.reason) active &= ~(1u << c);
+      beta[c] = h[c];
+    }
+    i++;
+  }
 }
 
 }  // namespace geneo

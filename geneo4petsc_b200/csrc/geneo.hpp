@@ -154,6 +154,15 @@ class GeneoPC {
   void initial_guess(const double* b, double* x0);        // x0 = Q b (efficient hybrid) or 0 (src/geneo.cpp:1601-1607)
   KspResult solve_cg(const double* b, double* x, double rtol, double atol, double dtol, int maxIt);
   KspResult solve_gmres(const double* b, double* x, double rtol, double atol, double dtol, int maxIt, int restart);
+  // Blocks of k right-hand sides (PCMatApply / KSPMatSolve), device pointers, column-major with leading dimensions >= nLoc.
+  // 8 columns at a time go through one pass over the level-1 factors (the 8-column solve kernel); k need not be a multiple
+  // of 8 (the last chunk is zero-padded).  Rows nLoc..ld-1 of the outputs are not written.
+  // apply_block: Y = M^-1 X, every variant apply() supports; X is not written.
+  void apply_block(int k, const double* X, int64_t ldx, double* Y, int64_t ldy);
+  // solve_cg_block: lock-step (pseudo-block) CG.  Every column runs solve_cg's recurrence from initial_guess()'s x0 (which
+  // it computes itself) with its own convergence test; a column that stops is frozen.  X receives the solutions.
+  std::vector<KspResult> solve_cg_block(int k, const double* B, int64_t ldb, double* X, int64_t ldx, double rtol, double atol,
+                                        double dtol, int maxIt);
   double dot(const double* x, const double* y);
   double norm(const double* x) { return std::sqrt(dot(x, x)); }
   // algorithmic bytes of one PC apply (SURVEY.md 8d) and of its dominant kernel family (factor sweeps)
@@ -197,6 +206,18 @@ class GeneoPC {
   DevBuf<double> dAll;
   DevBuf<int64_t> pullPtr, pullPos;
   int64_t nAll = 0;
+  // row-major 8-column blocks of the block apply, allocated on the first block call and kept (re-sized when a setup changes
+  // nAll / nLoc): the caller's columns in and out (bIn, bOut), the hybrid variants' intermediates (bT1, bT2), the
+  // concatenated subdomain blocks (bXall, bYall), the coarse vectors Z^T X and E^-1 Z^T X (bW, bW2)
+  DevBuf<double> bIn, bOut, bT1, bT2, bXall, bYall, bW, bW2;
+  void ensure_block();
+  void level1_8(double* x, double* y, bool addQ);  // x, y: nLoc x 8; the ghost rows of x are refreshed
+  void applyQ8(double* x, double* y);               // y may be x
+  void apply8(double* x, double* y);                // y != x
+  void mult8(double* x, double* y);                 // owned rows of y = A x
+  void mult_sub8(double* x, const double* b, double* y);  // owned rows of y = b - A x
+  void coarse8();                                    // bW2 = E^-1 Z^T bXall (nE x 8, allreduced over the ranks)
+  void cg8(const double* b, double* x, unsigned active, double rtol, double atol, double dtol, int maxIt, KspResult* res);
   std::vector<cudaStream_t> streams;
   std::vector<cudaEvent_t> events;
   cudaEvent_t evFork = nullptr;

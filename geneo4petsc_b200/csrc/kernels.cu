@@ -519,6 +519,85 @@ __global__ void k_update_robin(int n, const int64_t* __restrict__ ptr, const int
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// blocks of 8 right-hand sides.  Element t of a row-major n x 8 block is column t & 7; every grid stride below is a multiple
+// of 8, so a thread stays on the column threadIdx.x & 7.
+// ---------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ double coef_of(const Coef8& a, int c) {  // a.v[c] without dynamic indexing (no local memory)
+  double v = 0.;
+#pragma unroll
+  for (int q = 0; q < 8; q++) v = q == c ? a.v[q] : v;
+  return v;
+}
+__global__ void k_pack_cols8(int64_t n, int nc, const double* __restrict__ X, int64_t ldx, double* __restrict__ B) {
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n * 8; t += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(t & 7);
+    B[t] = c < nc ? X[c * ldx + (t >> 3)] : 0.;
+  }
+}
+__global__ void k_unpack_cols8(int64_t n, int nc, const double* __restrict__ B, double* __restrict__ Y, int64_t ldy) {
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < n * 8; t += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(t & 7);
+    if (c < nc) Y[c * ldy + (t >> 3)] = B[t];
+  }
+}
+__global__ void k_pull_sum8(int n, const int64_t* __restrict__ ptr, const int64_t* __restrict__ pos, const double* __restrict__ t,
+                            double* __restrict__ y) {
+  for (int64_t u = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; u < (int64_t)n * 8; u += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t g = u >> 3;
+    const int c = (int)(u & 7);
+    double s = 0.;
+    for (int64_t e = ptr[g]; e < ptr[g + 1]; e++) s += __ldg(t + pos[e] * 8 + c);
+    y[u] = s;
+  }
+}
+// out[c] += sum x_c y_c (and out[8 + c] += sum z_c z_c): lanes l, l ^ 8, l ^ 16, l ^ 24 share a column
+template <bool ZZ>
+__global__ void __launch_bounds__(256) k_dot_cols8(int64_t tot, const double* __restrict__ x, const double* __restrict__ y,
+                                                   const double* __restrict__ z, double* out) {
+  __shared__ double sh[2][8][8];
+  double a = 0., b = 0.;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < tot; t += (int64_t)gridDim.x * blockDim.x) {
+    a += x[t] * y[t];
+    if (ZZ) {
+      const double zz = z[t];
+      b += zz * zz;
+    }
+  }
+  a += __shfl_xor_sync(0xffffffffu, a, 8);
+  a += __shfl_xor_sync(0xffffffffu, a, 16);
+  if (ZZ) {
+    b += __shfl_xor_sync(0xffffffffu, b, 8);
+    b += __shfl_xor_sync(0xffffffffu, b, 16);
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (lane < 8) { sh[0][warp][lane] = a; sh[1][warp][lane] = b; }
+  __syncthreads();
+  if (threadIdx.x < 8) {
+    double sa = 0., sb = 0.;
+    for (int w = 0; w < (int)(blockDim.x >> 5); w++) { sa += sh[0][w][threadIdx.x]; sb += sh[1][w][threadIdx.x]; }
+    atomicAdd(out + threadIdx.x, sa);
+    if (ZZ) atomicAdd(out + 8 + threadIdx.x, sb);
+  }
+}
+__global__ void k_cg_update8(int64_t tot, Coef8 a, unsigned mask, const double* __restrict__ p, const double* __restrict__ w,
+                             double* __restrict__ x, double* __restrict__ r) {
+  const int c = threadIdx.x & 7;
+  if (!((mask >> c) & 1u)) return;
+  const double ac = coef_of(a, c);
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < tot; t += (int64_t)gridDim.x * blockDim.x) {
+    x[t] += ac * p[t];
+    r[t] -= ac * w[t];
+  }
+}
+__global__ void k_aypx8(int64_t tot, Coef8 b, unsigned mask, const double* __restrict__ z, double* __restrict__ p) {
+  const int c = threadIdx.x & 7;
+  if (!((mask >> c) & 1u)) return;
+  const double bc = coef_of(b, c);
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < tot; t += (int64_t)gridDim.x * blockDim.x)
+    p[t] = z[t] + bc * p[t];
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -751,6 +830,42 @@ void update_sell_add(int64_t nnz, const int64_t* slot, const double* neu, SellMa
 void update_robin(int n, const int64_t* ptr, const int* idx, const double* d, const double* dir, const double* neu, double optim,
                   double* rob, cudaStream_t st) {
   k_update_robin<<<GENEO_TICK(grid_for(n, 256)), 256, 0, st>>>(n, ptr, idx, d, dir, neu, optim, rob);
+  CUDA_CHECK(cudaGetLastError());
+}
+
+void pack_cols8(int64_t n, int nc, const double* X, int64_t ldx, double* B, cudaStream_t st) {
+  if (n == 0) return;
+  k_pack_cols8<<<GENEO_TICK(grid_for(n * 8, 256)), 256, 0, st>>>(n, nc, X, ldx, B);
+  CUDA_CHECK(cudaGetLastError());
+}
+void unpack_cols8(int64_t n, int nc, const double* B, double* Y, int64_t ldy, cudaStream_t st) {
+  if (n == 0) return;
+  k_unpack_cols8<<<GENEO_TICK(grid_for(n * 8, 256)), 256, 0, st>>>(n, nc, B, Y, ldy);
+  CUDA_CHECK(cudaGetLastError());
+}
+void pull_sum8(int n, const int64_t* ptr, const int64_t* pos, const double* t, double* y, cudaStream_t st) {
+  if (n == 0) return;
+  k_pull_sum8<<<GENEO_TICK(grid_for((int64_t)n * 8, 256)), 256, 0, st>>>(n, ptr, pos, t, y);
+  CUDA_CHECK(cudaGetLastError());
+}
+void dot_cols8(int n, const double* x, const double* y, const double* z, double* out, cudaStream_t st) {
+  CUDA_CHECK(cudaMemsetAsync(out, 0, (z ? 16 : 8) * sizeof(double), st));
+  if (n == 0) return;
+  const int64_t tot = (int64_t)n * 8;
+  if (z) k_dot_cols8<true><<<GENEO_TICK(grid_for(tot, 256, 4)), 256, 0, st>>>(tot, x, y, z, out);
+  else k_dot_cols8<false><<<GENEO_TICK(grid_for(tot, 256, 4)), 256, 0, st>>>(tot, x, y, nullptr, out);
+  CUDA_CHECK(cudaGetLastError());
+}
+void cg_update8(int n, Coef8 a, unsigned mask, const double* p, const double* w, double* x, double* r, cudaStream_t st) {
+  if (n == 0 || mask == 0) return;
+  const int64_t tot = (int64_t)n * 8;
+  k_cg_update8<<<GENEO_TICK(grid_for(tot, 256)), 256, 0, st>>>(tot, a, mask, p, w, x, r);
+  CUDA_CHECK(cudaGetLastError());
+}
+void aypx8(int n, Coef8 b, unsigned mask, const double* z, double* p, cudaStream_t st) {
+  if (n == 0 || mask == 0) return;
+  const int64_t tot = (int64_t)n * 8;
+  k_aypx8<<<GENEO_TICK(grid_for(tot, 256)), 256, 0, st>>>(tot, b, mask, z, p);
   CUDA_CHECK(cudaGetLastError());
 }
 

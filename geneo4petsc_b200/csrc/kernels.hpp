@@ -23,7 +23,8 @@ struct SellMatrix {
 void sell_spmv(const SellMatrix& A, const double* x, double* y, cudaStream_t st);              // y = A x
 void sell_spmv_sub(const SellMatrix& A, const double* x, const double* b, double* y, cudaStream_t st);  // y = b - A x
 
-// Y[:, 0:8] = A X[:, 0:8] (row-major blocks, ld 8) -- used by the coarse operator assembly W = A (R_j^T Z_j)
+// Y[:, 0:8] = A X[:, 0:8] (row-major blocks, ld 8) -- used by the coarse operator assembly W = A (R_j^T Z_j) and the block
+// PC apply / block CG
 void sell_spmm8(const SellMatrix& A, const double* X, double* Y, cudaStream_t st);
 
 struct CsrDev {
@@ -61,6 +62,21 @@ void pull_sum(int n, const int64_t* ptr, const int64_t* pos, const double* t, do
 // out[k*8 + c] = G[idx[k]*8 + c]
 void scatter_rows8(int n, const int* idx, const double* Z, int ldz, int c0, int nc, double* G, cudaStream_t st);
 void gather_rows8(int n, const int* idx, const double* G, double* out, cudaStream_t st);
+
+// ---- blocks of 8 right-hand sides (GeneoPC::apply_block / solve_cg_block): row-major n x 8 blocks ---------------------
+// B[i*8 + c] = X[c*ldx + i] for c < nc, 0 for nc <= c < 8 (column-major with leading dimension ldx -> row-major block)
+void pack_cols8(int64_t n, int nc, const double* X, int64_t ldx, double* B, cudaStream_t st);
+// Y[c*ldy + i] = B[i*8 + c] for c < nc (rows i >= n of Y are not written)
+void unpack_cols8(int64_t n, int nc, const double* B, double* Y, int64_t ldy, cudaStream_t st);
+// y[g*8 + c] = sum_{e in [ptr[g],ptr[g+1])} t[pos[e]*8 + c]   (pull_sum per column, same order)
+void pull_sum8(int n, const int64_t* ptr, const int64_t* pos, const double* t, double* y, cudaStream_t st);
+// per-column dots over n rows (out zeroed by the call): out[c] = x_c . y_c ; with z: also out[8 + c] = z_c . z_c
+void dot_cols8(int n, const double* x, const double* y, const double* z, double* out, cudaStream_t st);
+struct Coef8 { double v[8]; };  // one coefficient per column, passed by value
+// columns c with bit c of mask set: x_c += a_c p_c, r_c -= a_c w_c
+void cg_update8(int n, Coef8 a, unsigned mask, const double* p, const double* w, double* x, double* r, cudaStream_t st);
+// columns c with bit c of mask set: p_c = z_c + b_c p_c
+void aypx8(int n, Coef8 b, unsigned mask, const double* z, double* p, cudaStream_t st);
 
 // ---- tall-skinny dense --------------------------------------------------------------------------------------------
 // G[p x q] (row-major, ldg) += X[:,0:p]^T Y[:,0:q]   (n rows; caller zeroes G)

@@ -82,6 +82,15 @@ int geneo_pc_setup(geneo_pc_t pc, geneo_problem_t p);
 int geneo_pc_apply(geneo_pc_t pc, const double* x, double* y);
 int geneo_pc_apply_device(geneo_pc_t pc, const double* dx, double* dy);     /* same with device pointers            */
 int geneo_pc_apply_q_device(geneo_pc_t pc, const double* dx, double* dy);   /* applyQ, :1435-1542                   */
+/* PCMatApply: Y = M^-1 X for k >= 1 columns, every variant geneo_pc_apply supports (applyGenEOPC, :2051-2098, column by
+ * column).  X and Y are column-major (PETSc MATDENSE) with leading dimensions ldx, ldy >= the vector length (nbDof, or
+ * nLoc of geneo_pc_local_sizes on a multi-GPU PC, where the call is collective with local [owned | ghost] columns).
+ * 8 columns go through one pass over the level-1 factors; k need not be a multiple of 8.  X is not modified; rows
+ * between the vector length and ldy of Y are not written.  Each column agrees with geneo_pc_apply to rounding (the
+ * 8-column kernels sum in another order).  Fails with a message when k < 1, before setup ("without context"), or when a
+ * leading dimension is below the vector length. */
+int geneo_pc_apply_block(geneo_pc_t pc, int k, const double* X, int64_t ldx, double* Y, int64_t ldy);
+int geneo_pc_apply_block_device(geneo_pc_t pc, int k, const double* dX, int64_t ldx, double* dY, int64_t ldy);
 /* PCSetUp again with an unchanged non-zero pattern: every factorization, eigen-solve, Z and E recomputed from the
  * matrices already resident in HBM (no host analysis, no upload).  setUpGenEOPC is re-entered the same way when PETSc
  * flags the operator as changed (src/geneo.cpp:1672-1843). */
@@ -157,6 +166,15 @@ int geneo_ksp_solve(geneo_pc_t pc, const char* ksp, const double* b, double* x, 
                     int maxIt, int restart, int64_t out[3], double* rnorm, double* history, int histCap);
 int geneo_ksp_solve_device(geneo_pc_t pc, const char* ksp, const double* db, double* dx, double rtol, double atol,
                            double dtol, int maxIt, int restart, int64_t out[3], double* rnorm, double* history, int histCap);
+/* KSPMatSolve with KSPCG: k >= 1 right-hand sides B (column-major, ldb) solved in lock step, 8 columns per block SpMV and
+ * block PC apply (pseudo-block CG).  Every column runs geneo_ksp_solve's CG recurrence -- same initial guess, reference
+ * norm, convergence test and breakdown checks -- and stops on its own; X (column-major, ldx) receives the solutions.
+ * ksp must be "cg" (block GMRES is not provided).  out[2 j] = iterations, out[2 j + 1] = reason, rnorm[j] = final
+ * preconditioned residual norm of column j (either may be NULL).  Argument checks as geneo_pc_apply_block, ksp first. */
+int geneo_ksp_solve_block(geneo_pc_t pc, const char* ksp, int k, const double* B, int64_t ldb, double* X, int64_t ldx,
+                          double rtol, double atol, double dtol, int maxIt, int64_t* out, double* rnorm);
+int geneo_ksp_solve_block_device(geneo_pc_t pc, const char* ksp, int k, const double* dB, int64_t ldb, double* dX, int64_t ldx,
+                                 double rtol, double atol, double dtol, int maxIt, int64_t* out, double* rnorm);
 const char* geneo_ksp_reason_name(int reason);
 
 /* ------------------------------------------------------------------------------------------------------------------
